@@ -2,6 +2,7 @@
 """Benchmark of the hot path: med3ddram (ResNet-34) + dRAM inference on synthetic 256^3 CT volumes.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--size 256] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one pass of the device-resident hot path (SURVEY §8d) over one batch of B volumes per GPU:
@@ -28,6 +29,7 @@ import sys
 import time
 from argparse import Namespace
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -253,6 +255,26 @@ def max_over_ranks(value, world, device):
     t = torch.tensor([value], dtype=torch.float64, device=device)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     return float(t.item())
+
+
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Writes every tensor of `arrays` as <out_dir>/<name>.npy, float64 kept, anything else as float32, so that two
+    builds can be compared output for output.  Each array gets an equal share of DUMP_BYTES; one larger than its share
+    is written as a fixed sample, 1-D: its values at the flat indices
+    np.unique(np.random.default_rng(seed).integers(0, numel, share // itemsize)), which depend only on numel."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 128  # less the .npy header
+    for name, t in arrays.items():
+        dtype = torch.float64 if t.dtype == torch.float64 else torch.float32
+        itemsize = 8 if dtype == torch.float64 else 4
+        t = t.detach()
+        if t.numel() * itemsize > share:
+            idx = np.unique(np.random.default_rng(seed).integers(0, t.numel(), share // itemsize))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.to(dtype).cpu().numpy())
 
 
 # --------------------------------------------------------------------------------------------
@@ -603,7 +625,15 @@ def main():
     ap.add_argument("--mode", default="infer", choices=["infer", "train"],
                     help="infer (default): BASELINE.json's headline metric; train: one data-parallel training step "
                          "(BASELINE config 5; additional line, not the headline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one returned (dRAM maps and percentages of rank "
+                         "0's volumes) as DIR/<name>.npy, at most 64 MB in all: a larger map is a fixed, seeded sample "
+                         "(see dump_outputs); default inference arm only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "infer"):
+        ap.error("--dump-outputs applies to the default inference arm (--impl ours --mode infer)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     sink = _StdoutToStderr()
     if args.impl == "reference":
@@ -649,6 +679,8 @@ def main():
     barrier(world)
     ms_total = max_over_ranks(e0.elapsed_time(e1), world, device)
     clocks = sampler.stop(skip=first_sample) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)  # predict_step_from_hu allocates its outputs: `out` is the last step's
     ms_per_step = ms_total / args.steps
     value = world * B / (ms_per_step * 1e-3)
     launches_per_step = len(eng.steps) + 3 + 2  # K8 statistics + finalize + apply; the recorded steps; K7 + finalize

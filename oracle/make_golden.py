@@ -1,6 +1,6 @@
 """Generates tests/golden/* by running the UNMODIFIED reference on CPU.  TEST INFRASTRUCTURE.
 
-    python -m oracle.make_golden            (from the repo root, where /root/reference is mounted)
+    DRAM_REFERENCE_DIR=<upstream checkout> python -m oracle.make_golden      (from the repo root)
 
 Every fixture records the seeds/dims that regenerate its inputs with oracle/synthetic.py, a
 fingerprint of the weights, and the reference's outputs.  Nothing here is imported by product code;

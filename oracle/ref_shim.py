@@ -4,8 +4,8 @@ The reference needs pytorch_lightning, hydra, omegaconf, SimpleITK, matplotlib a
 of which is installed in this image; they are only used for orchestration, plotting and file I/O,
 never for arithmetic on the hot path.  `load()` plants minimal stand-ins in sys.modules, puts the
 reference checkout on sys.path, chdir()s into it (utils.py:84 opens ./conf/<name>.yaml relative to
-the cwd) and imports its modules.  Works only where the checkout exists (this container, not the
-GPU box); used by make_golden.py and by the parity-pinning tests that skip when it is absent.
+the cwd) and imports its modules.  Works only where DRAM_REFERENCE_DIR names a checkout of the
+upstream project; used by make_golden.py and by the parity-pinning tests that skip without one.
 """
 import contextlib
 import enum
@@ -14,14 +14,14 @@ import os
 import sys
 import types
 
-REF_DIR = os.environ.get("DRAM_REFERENCE_DIR", "/root/reference")
+REF_DIR = os.environ.get("DRAM_REFERENCE_DIR", "")
 
 _REF_MODULES = ["med3d", "models", "utils", "dataset", "base", "functional", "intensity_transforms",
                 "spatial_transforms", "metrics", "sampler", "data_sampler", "confusion_matrix"]
 
 
 def available():
-    return os.path.isfile(os.path.join(REF_DIR, "med3d.py"))
+    return bool(REF_DIR) and os.path.isfile(os.path.join(REF_DIR, "med3d.py"))
 
 
 def _module(name, **attrs):
@@ -104,7 +104,7 @@ def load():
     if _loaded is not None:
         return _loaded
     if not available():
-        raise FileNotFoundError(f"reference checkout not found at {REF_DIR}")
+        raise FileNotFoundError(f"no reference checkout: set DRAM_REFERENCE_DIR (now {REF_DIR!r})")
     for name in _REF_MODULES:
         if name in sys.modules and not getattr(sys.modules[name], "__file__", "").startswith(REF_DIR):
             raise RuntimeError(f"module name clash: '{name}' is already imported from elsewhere")

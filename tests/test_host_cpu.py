@@ -553,6 +553,45 @@ def test_bench_reference_arm_prints_the_contract_line(tmp_path):
     assert other.returncode == 0 and other.stdout.strip() == ""
 
 
+def test_bench_dump_outputs_budget_and_sample(tmp_path):
+    """`bench.py --dump-outputs`: float32 (float64 kept) .npy per output, at most 64 MB in all, arrays too large for
+    their share written as the same seeded sample on every run; bad arguments are refused before any work."""
+    import importlib.util
+
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    # every map holds its own flat index (exact in float32 below 2^24), so a sample shows which voxels it took
+    shape = (2, 1, 160, 160, 160)
+    n = int(np.prod(shape))
+    g = torch.Generator().manual_seed(0)
+    arrays = {"cle_dense_outs": torch.arange(n, dtype=torch.float32).reshape(shape),
+              "pse_dense_outs": torch.arange(n, dtype=torch.float64).reshape(shape),
+              "cle_precentages": torch.rand(2, generator=g).half(), "pse_precentages": torch.rand(2, generator=g).double()}
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(f"{k}.npy" for k in arrays)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64_000_000
+    loaded = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    for f in files:
+        assert np.array_equal(loaded[f[:-4]], np.load(tmp_path / "b" / f))
+    assert loaded["pse_precentages"].dtype == np.float64 and np.array_equal(loaded["pse_precentages"], arrays["pse_precentages"].numpy())
+    assert loaded["cle_precentages"].dtype == np.float32
+    assert np.array_equal(loaded["cle_precentages"], arrays["cle_precentages"].float().numpy())
+    for k, dtype in (("cle_dense_outs", np.float32), ("pse_dense_outs", np.float64)):
+        s = loaded[k]
+        assert s.dtype == dtype and s.ndim == 1 and 0 < s.size < n, (k, s.dtype, s.shape)
+        assert np.array_equal(s, np.round(s)) and s[0] >= 0 and s[-1] < n  # values of the array, i.e. voxel indices
+        assert (np.diff(s) > 0).all()                                      # distinct voxels in flat order
+        assert s[0] < n // 100 and s[-1] > n - n // 100                    # spread over the whole map
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "c")]):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + bad, capture_output=True, text=True,
+                             cwd=str(tmp_path), timeout=600)
+        assert res.returncode == 2 and res.stdout == "", (bad, res.stderr[-500:])
+    assert not (tmp_path / "c").exists()
+
+
 def test_inference_dataset_has_no_cpu_path(tmp_path):
     """Without a CUDA device the dataset reads the files and then refuses: the pre-steps of dataset.py:66-83 exist on
     the GPU only (their CPU restatement is the oracle's, not the product's)."""

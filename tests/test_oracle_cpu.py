@@ -1,5 +1,5 @@
 """Pins the CPU oracle (oracle/*.py) against golden vectors produced by the unmodified reference
-(oracle/make_golden.py) and — where /root/reference is mounted — against the live reference.
+(oracle/make_golden.py) and — where DRAM_REFERENCE_DIR names an upstream checkout — against the live reference.
 No GPU needed."""
 import glob
 import json
@@ -15,6 +15,18 @@ from oracle import ref_shim, synthetic
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 FORWARD_FIXTURES = sorted(glob.glob(os.path.join(GOLDEN, "forward_*.pt")))
+REF_SKIP = "needs DRAM_REFERENCE_DIR: a checkout of the upstream project"
+
+
+@pytest.fixture(autouse=True)
+def _eight_cpu_threads():
+    """The goldens were computed multi-threaded.  With 4 threads or fewer ATen's CPU kernels sum in another order, and
+    that moves the saturating reference-init maps and the gradient of a bias that feeds train-mode BatchNorm (zero up
+    to rounding) past the tolerances.  So the thread count is fixed here, not left to the host or an earlier test."""
+    before = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(before)
 
 
 def test_state_layout_matches_reference_modules():
@@ -162,13 +174,13 @@ LIVE_CASES = [
 ]
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not mounted")
+@pytest.mark.skipif(not ref_shim.available(), reason=REF_SKIP)
 @pytest.mark.parametrize("arch,dims,batch,with_mask", LIVE_CASES)
 def test_oracle_against_live_reference(arch, dims, batch, with_mask):
     """The oracle's forward against the unmodified reference module executed here (through oracle/ref_shim.py) on the
     same seeded weights and inputs: bit-identical dense maps and scores for all six architectures, ragged sizes,
-    batches of two and the lungs=None path.  (Only runs where /root/reference is mounted; the committed golden vectors
-    carry the same pin to the GPU box.)"""
+    batches of two and the lungs=None path.  (Only runs with DRAM_REFERENCE_DIR set; these cases have no golden
+    vectors, the forward goldens above cover other shapes to 2e-5.)"""
     sd = synthetic.make_state_dict(arch, seed=3, calib_dims=dims)
     ref = ref_shim.model(arch)
     ref.load_state_dict(sd)
@@ -186,7 +198,7 @@ def test_oracle_against_live_reference(arch, dims, batch, with_mask):
         assert torch.equal(a, b)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not mounted")
+@pytest.mark.skipif(not ref_shim.available(), reason=REF_SKIP)
 @pytest.mark.parametrize("arch,dims,batch", [("med3ddram", (16, 24, 32), 3), ("med3ddram50", (16, 16, 24), 1),
                                               ("med3ddram18", (24, 16, 16), 2)])
 def test_predict_step_oracle_against_live_reference(arch, dims, batch):
@@ -220,7 +232,7 @@ def test_predict_step_oracle_against_live_reference(arch, dims, batch):
         module._ratio_to_label(want["pse_precentages"], pse_map).tolist()
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not mounted")
+@pytest.mark.skipif(not ref_shim.available(), reason=REF_SKIP)
 @pytest.mark.parametrize("scan_dims,target", [((40, 48, 56), (24, 32, 40)), ((30, 36, 44), (32, 48, 40)),
                                                ((33, 47, 51), (16, 47, 64))])
 def test_transforms_oracle_against_live_reference(scan_dims, target):
@@ -278,7 +290,7 @@ def test_label_bands_follow_the_ratio_maps():
         assert torch.equal(T.label_bands(lab, mapping), want)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not mounted")
+@pytest.mark.skipif(not ref_shim.available(), reason=REF_SKIP)
 @pytest.mark.parametrize("arch,dims,batch", [("med3ddram50", (16, 16, 16), 2), ("med3ddram", (16, 16, 24), 1)])
 def test_training_oracle_against_live_reference(arch, dims, batch):
     """The training oracle (train-mode BatchNorm, detached shortcut A, the reference's loss) against one training step

@@ -1,6 +1,8 @@
 """predict_step, the GPU inference transform and the processor CLI against the reference goldens / the oracle."""
 import json
 import os
+import subprocess
+import sys
 from argparse import Namespace
 
 import numpy as np
@@ -215,3 +217,34 @@ def test_device_prefetcher_delivers_every_batch_intact(cuda, lib, shape, streams
         seen += 1
     assert seen == 5
     assert list(DevicePrefetcher(iter([]), cuda)) == []
+
+
+def test_bench_dump_outputs_are_the_timed_path_outputs(cuda, lib, tmp_path):
+    """`bench.py --steps K --dump-outputs DIR`: the line reports K timed steps, and the dump holds what the timed path
+    (predict_step_from_hu on bench.py's seeded volumes and weights) returns, the same for any K."""
+    import importlib.util
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    dims, batch = (32, 32, 32), 2
+    with torch.random.fork_rng(devices=[cuda]):  # build_module seeds the global generator
+        module = bench.build_module(cuda)
+    want = {k: v.float().cpu().numpy() for k, v in
+            module.predict_step_from_hu(*bench.make_volumes(batch, dims, cuda, seed=0)).items()}
+    del module
+    for steps in (1, 3):
+        out_dir = tmp_path / f"steps{steps}"
+        cmd = [sys.executable, os.path.join(root, "bench.py"), "--size", "32", "--batch", str(batch), "--steps", str(steps),
+               "--warmup", "1", "--no-cpu-baseline", "--no-train-field", "--no-yardstick", "--dump-outputs", str(out_dir)]
+        res = subprocess.run(cmd, capture_output=True, text=True, cwd=str(tmp_path), timeout=900)
+        assert res.returncode == 0, res.stderr[-2000:]
+        assert json.loads(res.stdout)["steps"] == steps
+        assert sorted(os.listdir(out_dir)) == sorted(f"{k}.npy" for k in want)
+        for k, ref in want.items():
+            got = np.load(out_dir / f"{k}.npy")
+            assert got.dtype == np.float32 and got.shape == ref.shape, (k, got.dtype, got.shape)
+            np.testing.assert_allclose(got, ref, rtol=1e-5, atol=1e-6, err_msg=k)
+            if k.endswith("dense_outs"):
+                assert np.array_equal(got == 0, ref == 0), k
