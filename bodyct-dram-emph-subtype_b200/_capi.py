@@ -77,6 +77,8 @@ SIGNATURES = {
     "dram_dram_workspace_bytes": (_sz, [_i32]),
     "dram_dram_upsample_mask": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32,
                                           _i32, _i32, _i32, _i32, _vp]),
+    "dram_lobe_workspace_bytes": (_sz, [_i32, _i64]),
+    "dram_lobe_sums": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _vp]),
     "dram_preprocess_workspace_bytes": (_sz, []),
     "dram_window_standardize": (C.c_int, [_vp, _vp, _vp, _vp, _i64, C.c_float, C.c_float, _vp]),
     "dram_preprocess_workspace_bytes_n": (_sz, [_i32]),
@@ -85,6 +87,7 @@ SIGNATURES = {
     "dram_window_lut": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i64, C.c_float, C.c_float, _vp]),
     "dram_resize_image": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "dram_resize_mask": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
+    "dram_resize_labels": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "dram_mask_bbox": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp]),
     "dram_lung_crop_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "dram_lung_crop": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),

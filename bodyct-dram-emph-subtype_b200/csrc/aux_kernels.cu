@@ -55,6 +55,21 @@ __device__ __forceinline__ double warp_sum(double v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
+// Block-wide sums of `a` and `b` in one pair of barriers; results valid in thread 0.
+__device__ __forceinline__ void block_sum2(double &a, double &b, double2 *scratch) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  a = warp_sum(a);
+  b = warp_sum(b);
+  __syncthreads();
+  if (lane == 0) scratch[warp] = make_double2(a, b);
+  __syncthreads();
+  if (warp == 0) {
+    const int nw = (blockDim.x + 31) >> 5;
+    const double2 v = lane < nw ? scratch[lane] : make_double2(0.0, 0.0);
+    a = warp_sum(v.x);
+    b = warp_sum(v.y);
+  }
+}
 // Block-wide sum of `v`; result valid in thread 0.  `scratch` has >= 32 doubles.
 __device__ __forceinline__ double block_sum(double v, double *scratch) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -716,6 +731,174 @@ __global__ void dram_finalize_kernel(const double *__restrict__ sums, float *__r
 }
 
 // ---------------------------------------------------------------------------------------
+// K7l per-label dRAM sums: for every label k of a uint8 label volume, the voxel count and the sums of both
+// dRAM maps over the `ess` voxels labelled k.  Bit-reproducible without floating-point atomics:
+//   partial: grid (P, n).  A CTA walks tiles p, p+P, ... of its sample.  Per tile every thread holds 4 x 16
+//            labels and ess bytes in registers (16-byte loads, or byte loads on the scalar path), adds its runs of
+//            equal labels to shared integer counts and marks the labels that have ess voxels in a 256-bit set;
+//            then, for each marked label in increasing order, one fixed-tree block sum (fp64) of the map values
+//            (read only at ess voxels) that thread 0 adds to the CTA's accumulator.  Each CTA writes all 256
+//            entries of its partial (zeros included).
+//   finish:  grid (8, n), 32 labels per CTA; warp w adds partials w, w+8, ... in order, then warps 0..7 in order.
+// ---------------------------------------------------------------------------------------
+static constexpr int LOBE_THREADS = 256;
+static constexpr int LOBE_VECS = 4;                                   // 16-voxel vectors per thread and tile
+static constexpr int LOBE_TILE = LOBE_THREADS * LOBE_VECS * 16;       // 16384 voxels
+static constexpr int LOBE_LABELS = 256;
+
+__device__ __forceinline__ unsigned byte_of(const uint32_t (&w)[LOBE_VECS * 4], int j, int k) {
+  return (w[j * 4 + (k >> 2)] >> (8 * (k & 3))) & 0xffu;
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(LOBE_THREADS)
+lobe_sums_partial_kernel(const float *__restrict__ map0, const float *__restrict__ map1, const uint8_t *__restrict__ ess,
+                         const uint8_t *__restrict__ labels, double *__restrict__ psum, uint32_t *__restrict__ pcnt,
+                         int64_t count) {
+  __shared__ uint32_t cnt[LOBE_LABELS];
+  __shared__ double acc0[LOBE_LABELS], acc1[LOBE_LABELS];
+  __shared__ uint32_t marked[LOBE_LABELS / 32];
+  __shared__ double2 scratch[32];
+  const int t = threadIdx.x, P = gridDim.x;
+  const int64_t base = (int64_t)blockIdx.y * count;
+  const float *m0 = map0 + base, *m1 = map1 + base;
+  const uint8_t *es = ess + base, *lb = labels + base;
+  cnt[t] = 0;
+  acc0[t] = 0.0;
+  acc1[t] = 0.0;
+  const int64_t tiles = (count + LOBE_TILE - 1) / LOBE_TILE;
+  for (int64_t tile = blockIdx.x; tile < tiles; tile += P) {
+    if (t < LOBE_LABELS / 32) marked[t] = 0;
+    __syncthreads();
+    const int64_t t0 = tile * LOBE_TILE;
+    uint32_t lw[LOBE_VECS * 4], ew[LOBE_VECS * 4];
+    int nv[LOBE_VECS];
+#pragma unroll
+    for (int j = 0; j < LOBE_VECS; ++j) {
+      const int64_t o = t0 + (int64_t)(j * LOBE_THREADS + t) * 16;
+      const int64_t left = count - o;
+      nv[j] = left <= 0 ? 0 : (left >= 16 ? 16 : (int)left);
+      if constexpr (VEC) {  // count % 16 == 0: a vector is whole or absent
+        const uint4 l4 = nv[j] ? __ldg(reinterpret_cast<const uint4 *>(lb + o)) : make_uint4(0, 0, 0, 0);
+        const uint4 e4 = nv[j] ? __ldg(reinterpret_cast<const uint4 *>(es + o)) : make_uint4(0, 0, 0, 0);
+        lw[j * 4 + 0] = l4.x; lw[j * 4 + 1] = l4.y; lw[j * 4 + 2] = l4.z; lw[j * 4 + 3] = l4.w;
+        ew[j * 4 + 0] = e4.x; ew[j * 4 + 1] = e4.y; ew[j * 4 + 2] = e4.z; ew[j * 4 + 3] = e4.w;
+      } else {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) lw[j * 4 + q] = ew[j * 4 + q] = 0;
+        for (int k = 0; k < nv[j]; ++k) {
+          lw[j * 4 + (k >> 2)] |= (uint32_t)__ldg(lb + o + k) << (8 * (k & 3));
+          ew[j * 4 + (k >> 2)] |= (uint32_t)(__ldg(es + o + k) != 0) << (8 * (k & 3));
+        }
+      }
+    }
+    // counts (runs of one label -> one shared atomic), the set of labels with ess voxels, and this thread's map sums
+    // over its ess voxels while they carry one label (all map loads of the tile in one burst, before any barrier)
+    unsigned cur = LOBE_LABELS, run = 0, last_marked = LOBE_LABELS, mine = LOBE_LABELS;
+    double a0 = 0.0, a1 = 0.0;
+    bool mixed = false;
+#pragma unroll
+    for (int j = 0; j < LOBE_VECS; ++j) {
+      const int64_t o = t0 + (int64_t)(j * LOBE_THREADS + t) * 16;
+#pragma unroll
+      for (int k = 0; k < 16; ++k) {
+        if (k < nv[j]) {
+          const unsigned lab = byte_of(lw, j, k);
+          if (lab != cur) {
+            if (run) atomicAdd(&cnt[cur], run);
+            cur = lab;
+            run = 0;
+          }
+          ++run;
+          if (byte_of(ew, j, k)) {
+            if (lab != last_marked) {
+              atomicOr(&marked[lab >> 5], 1u << (lab & 31));
+              last_marked = lab;
+            }
+            if (mine == LOBE_LABELS) mine = lab;
+            if (lab == mine) {
+              a0 += (double)__ldg(m0 + o + k);
+              a1 += (double)__ldg(m1 + o + k);
+            } else {
+              mixed = true;
+            }
+          }
+        }
+      }
+    }
+    if (run) atomicAdd(&cnt[cur], run);
+    __syncthreads();
+    for (int w = 0; w < LOBE_LABELS / 32; ++w) {
+      uint32_t set = marked[w];  // the same word in every thread: the loop below is uniform across the CTA
+      while (set) {
+        const int bit = __ffs(set) - 1;
+        set &= set - 1;
+        const unsigned label = (unsigned)(w * 32 + bit);
+        double s0 = label == mine ? a0 : 0.0, s1 = label == mine ? a1 : 0.0;
+        if (mixed) {  // ess voxels of several labels: sum this label's again, in the same voxel order
+          s0 = s1 = 0.0;
+#pragma unroll
+          for (int j = 0; j < LOBE_VECS; ++j) {
+            const int64_t o = t0 + (int64_t)(j * LOBE_THREADS + t) * 16;
+#pragma unroll
+            for (int k = 0; k < 16; ++k) {
+              if (k < nv[j] && byte_of(ew, j, k) && byte_of(lw, j, k) == label) {
+                s0 += (double)__ldg(m0 + o + k);
+                s1 += (double)__ldg(m1 + o + k);
+              }
+            }
+          }
+        }
+        block_sum2(s0, s1, scratch);
+        if (t == 0) {
+          acc0[label] += s0;
+          acc1[label] += s1;
+        }
+      }
+    }
+    __syncthreads();  // `marked` is reset for the next tile only after every thread has read it
+  }
+  __syncthreads();
+  const int64_t slot = (int64_t)blockIdx.y * P + blockIdx.x;
+  psum[(slot * 2 + 0) * LOBE_LABELS + t] = acc0[t];
+  psum[(slot * 2 + 1) * LOBE_LABELS + t] = acc1[t];
+  pcnt[slot * LOBE_LABELS + t] = cnt[t];
+}
+
+__global__ void __launch_bounds__(256)
+lobe_sums_finish_kernel(const double *__restrict__ psum, const uint32_t *__restrict__ pcnt, float *__restrict__ pct,
+                        int64_t *__restrict__ voxels, int n, int P) {
+  __shared__ double r0[8][32], r1[8][32];
+  __shared__ unsigned long long rc[8][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, b = blockIdx.y;
+  const int label = blockIdx.x * 32 + lane;
+  double s0 = 0.0, s1 = 0.0;
+  unsigned long long c = 0;
+  for (int p = warp; p < P; p += 8) {
+    const int64_t slot = (int64_t)b * P + p;
+    s0 += psum[(slot * 2 + 0) * LOBE_LABELS + label];
+    s1 += psum[(slot * 2 + 1) * LOBE_LABELS + label];
+    c += pcnt[slot * LOBE_LABELS + label];
+  }
+  r0[warp][lane] = s0;
+  r1[warp][lane] = s1;
+  rc[warp][lane] = c;
+  __syncthreads();
+  if (warp == 0) {
+    for (int w = 1; w < 8; ++w) {
+      s0 += r0[w][lane];
+      s1 += r1[w][lane];
+      c += rc[w][lane];
+    }
+    const int64_t o = (int64_t)b * LOBE_LABELS + label;
+    voxels[o] = (int64_t)c;
+    // the conversion of dram_finalize_kernel; 0 / 0 gives NaN for a label without voxels
+    pct[o] = (float)s0 / (float)c;
+    pct[(int64_t)n * LOBE_LABELS + o] = (float)s1 / (float)c;
+  }
+}
+
+// ---------------------------------------------------------------------------------------
 // K8 HU window + standardise: pass 1 accumulates sum and sum of squares of the windowed
 // values in fp64, pass 2 derives mean / unbiased std and writes (v - mean) / std in fp32.
 // ---------------------------------------------------------------------------------------
@@ -840,6 +1023,8 @@ __global__ void resize_image_kernel(const float *__restrict__ x, float *__restri
              ih.w1 * (iw.w0 * __ldg(r1 + iw.i0) + iw.w1 * __ldg(r1 + iw.i1));
   }
 }
+// KEEP = false: the mask rule (0/1 out); KEEP = true: the same voxel picked, its value kept (label volumes).
+template <bool KEEP>
 __global__ void resize_mask_kernel(const uint8_t *__restrict__ x, uint8_t *__restrict__ out,
                                    const int *__restrict__ d_idx, int H, int W, int D2, int H2, int W2) {
   const int64_t total = (int64_t)D2 * H2 * W2;
@@ -850,7 +1035,8 @@ __global__ void resize_mask_kernel(const uint8_t *__restrict__ x, uint8_t *__res
     const int xh = (int)(r % H2);
     const int xd = (int)(r / H2);
     const int zh = nearest_index(xh, H, H2), zw = nearest_index(xw, W, W2);
-    out[t] = x[((int64_t)__ldg(d_idx + xd) * H + zh) * W + zw] ? 1 : 0;
+    const uint8_t v = x[((int64_t)__ldg(d_idx + xd) * H + zh) * W + zw];
+    out[t] = KEEP ? v : (v ? 1 : 0);
   }
 }
 
@@ -1101,6 +1287,41 @@ extern "C" int dram_dram_upsample_mask(const float *dense0, const float *dense1,
   return DRAM_OK;
 }
 
+// CTAs per sample of the per-label sums: ~1024 in all, at least two tiles each.  A function of the shape only, so the
+// summation order (and with it every bit of the result) does not depend on the device.
+static int lobe_ctas(int32_t n, int64_t count) {
+  const int64_t tiles = ceil_div64(count, LOBE_TILE);
+  int64_t p = ceil_div64(tiles, 2);
+  const int64_t cap = n >= 1024 ? 1 : 1024 / n;
+  if (p > cap) p = cap;
+  return p < 1 ? 1 : (int)p;
+}
+
+extern "C" size_t dram_lobe_workspace_bytes(int32_t n, int64_t count) {
+  if (n <= 0 || count <= 0) return 0;
+  return (size_t)n * lobe_ctas(n, count) * LOBE_LABELS * (2 * sizeof(double) + sizeof(uint32_t));
+}
+
+extern "C" int dram_lobe_sums(const float *map0, const float *map1, const uint8_t *ess, const uint8_t *labels,
+                              float *pct, int64_t *voxels, void *workspace, int32_t n, int64_t count, void *stream) {
+  DRAM_REQUIRE(map0 && map1 && ess && labels && pct && voxels && workspace, "dram_lobe_sums: null pointer");
+  DRAM_REQUIRE(n > 0 && n <= 65535 && count > 0, "dram_lobe_sums: bad shape");
+  DRAM_REQUIRE(count < 0x7fffffffLL, "dram_lobe_sums: volume too large for 32-bit per-CTA counts");
+  DRAM_REQUIRE((uintptr_t)workspace % 8 == 0, "dram_lobe_sums: workspace must be 8-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int P = lobe_ctas(n, count);
+  double *psum = reinterpret_cast<double *>(workspace);
+  uint32_t *pcnt = reinterpret_cast<uint32_t *>(psum + (size_t)n * P * 2 * LOBE_LABELS);
+  const bool vec = (count % 16 == 0) && (((uintptr_t)ess | (uintptr_t)labels) % 16 == 0);
+  dim3 grid(P, n);
+  if (vec) lobe_sums_partial_kernel<true><<<grid, LOBE_THREADS, 0, st>>>(map0, map1, ess, labels, psum, pcnt, count);
+  else lobe_sums_partial_kernel<false><<<grid, LOBE_THREADS, 0, st>>>(map0, map1, ess, labels, psum, pcnt, count);
+  DRAM_CHECK_LAUNCH("lobe_sums_partial_kernel");
+  lobe_sums_finish_kernel<<<dim3(LOBE_LABELS / 32, n), 256, 0, st>>>(psum, pcnt, pct, voxels, n, P);
+  DRAM_CHECK_LAUNCH("lobe_sums_finish_kernel");
+  return DRAM_OK;
+}
+
 extern "C" size_t dram_preprocess_workspace_bytes(void) { return 2 * sizeof(double) + 2 * sizeof(float); }
 extern "C" size_t dram_preprocess_workspace_bytes_n(int32_t n) {
   return n > 0 ? (size_t)n * (2 * sizeof(double) + 2 * sizeof(float)) : 0;
@@ -1194,9 +1415,20 @@ extern "C" int dram_resize_mask(const uint8_t *x, uint8_t *out, const int32_t *d
   DRAM_REQUIRE(x && out && d_idx, "dram_resize_mask: null pointer");
   DRAM_REQUIRE(D > 0 && H > 0 && W > 0 && D2 > 0 && H2 > 0 && W2 > 0, "dram_resize_mask: bad shape");
   const int64_t total = (int64_t)D2 * H2 * W2;
-  resize_mask_kernel<<<stream_grid(total, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
+  resize_mask_kernel<false><<<stream_grid(total, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
       x, out, d_idx, H, W, D2, H2, W2);
   DRAM_CHECK_LAUNCH("resize_mask_kernel");
+  return DRAM_OK;
+}
+
+extern "C" int dram_resize_labels(const uint8_t *x, uint8_t *out, const int32_t *d_idx, int32_t D, int32_t H,
+                                  int32_t W, int32_t D2, int32_t H2, int32_t W2, void *stream) {
+  DRAM_REQUIRE(x && out && d_idx, "dram_resize_labels: null pointer");
+  DRAM_REQUIRE(D > 0 && H > 0 && W > 0 && D2 > 0 && H2 > 0 && W2 > 0, "dram_resize_labels: bad shape");
+  const int64_t total = (int64_t)D2 * H2 * W2;
+  resize_mask_kernel<true><<<stream_grid(total, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
+      x, out, d_idx, H, W, D2, H2, W2);
+  DRAM_CHECK_LAUNCH("resize_labels_kernel");
   return DRAM_OK;
 }
 

@@ -116,6 +116,20 @@ def _(dense0, dense1, ess, lungs, per_sample_denominator=False):
     return (dense0.new_empty((n, 1, D, H, W)), dense0.new_empty((n, 1, D, H, W)), dense0.new_empty((2, n)))
 
 
+@custom_op(f"{NS}::lobe_scores", mutates_args=(), device_types="cuda")
+def lobe_scores(cle: torch.Tensor, pse: torch.Tensor, ess: torch.Tensor,
+                labels: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Lesion percentages of both dRAM maps per label of a uint8 label volume (per lobe): (pct fp32 [2, B, 256],
+    voxels int64 [B, 256]), each label divided by its own voxel count."""
+    return ops.lobe_scores(cle, pse, ess, labels)
+
+
+@lobe_scores.register_fake
+def _(cle, pse, ess, labels):
+    B = labels.shape[0]
+    return (cle.new_empty((2, B, ops.LOBE_LABELS)), cle.new_empty((B, ops.LOBE_LABELS), dtype=torch.int64))
+
+
 # ------------------------------------------------------------------------------------------------ K8 / K8b
 @custom_op(f"{NS}::window_standardize", mutates_args=(), device_types="cuda")
 def window_standardize(hu: torch.Tensor, lo: float = -1150.0, hi: float = -300.0) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -165,4 +179,4 @@ def _(dram_map, crop, original_size):
 
 
 REGISTERED = ("conv3d", "stem_conv7", "maxpool3d", "upsample2x", "masked_pool", "dram_upsample_mask",
-              "window_standardize", "resize_image", "resize_mask", "heatmap_u8")
+              "window_standardize", "resize_image", "resize_mask", "heatmap_u8", "lobe_scores")

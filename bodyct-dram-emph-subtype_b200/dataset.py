@@ -29,15 +29,32 @@ def grow_bbox(bbox, shape, spacing, border):
     return out
 
 
+def labels_as_u8(lobe, uid):
+    """The lobe segmentation as a uint8 label volume: uint8 as it is; another integer (or bool) type when every value
+    lies in 0..255; anything else raises ValueError naming the scan."""
+    lobe = np.asarray(lobe)
+    if lobe.dtype == np.uint8:
+        return lobe
+    if lobe.dtype.kind not in "iub":
+        raise ValueError(f"{uid}: lobe labels of type {lobe.dtype} are not integers")
+    if lobe.size and (int(lobe.min()) < 0 or int(lobe.max()) > 255):
+        raise ValueError(f"{uid}: lobe labels span {int(lobe.min())}..{int(lobe.max())}, outside 0..255")
+    return lobe.astype(np.uint8)
+
+
 class SubtypingInference(torch.utils.data.Dataset):
     label_to_cle = {0: "absent", 1: "trace", 2: "mild", 3: "moderate", 4: "confluence", 5: "destructive"}
     label_to_pse = {0: "absent", 1: "mild", 2: "substantial"}
 
-    def __init__(self, scan_path, lobe_path, transforms=None, keep_sorted=True, crop_border=5, device=None):
+    def __init__(self, scan_path, lobe_path, transforms=None, keep_sorted=True, crop_border=5, device=None,
+                 lobe_labels=False):
+        """`lobe_labels=True`: every sample also carries `lobe_labels`, the uint8 label volume cropped like the masks
+        (for the per-lobe percentages)."""
         super().__init__()
         self.device = torch.device(device) if device is not None else getattr(transforms, "device", None)
         self.scan_path, self.lobe_path = scan_path, lobe_path
         self.keep_sorted, self.transforms, self.crop_border = keep_sorted, transforms, crop_border
+        self.lobe_labels = lobe_labels
         self.scan_files = sorted(glob.glob(os.path.join(scan_path, "*.mha")))
         self.lobe_files = sorted(glob.glob(os.path.join(lobe_path, "*.mha")))
         self.scan_meta_cache = {}
@@ -60,15 +77,18 @@ class SubtypingInference(torch.utils.data.Dataset):
 
         dev = self.device
         scan_d = torch.as_tensor(np.ascontiguousarray(scan)).to(torch.int16).to(dev, non_blocking=True)
-        lobe_d = torch.as_tensor(np.ascontiguousarray(lobe))
-        lobe_d = (lobe_d.to(torch.uint8) if lobe_d.dtype in (torch.uint8, torch.int8, torch.bool)
-                  else (lobe_d > 0).to(torch.uint8)).to(dev, non_blocking=True)
+        if self.lobe_labels:  # values kept: lung_crop takes labels > 0 itself
+            lobe_d = torch.as_tensor(np.ascontiguousarray(labels_as_u8(lobe, uid))).to(dev, non_blocking=True)
+        else:
+            lobe_d = torch.as_tensor(np.ascontiguousarray(lobe))
+            lobe_d = (lobe_d.to(torch.uint8) if lobe_d.dtype in (torch.uint8, torch.int8, torch.bool)
+                      else (lobe_d > 0).to(torch.uint8)).to(dev, non_blocking=True)
         bbox = ops.mask_bbox(lobe_d).cpu().tolist()
         if bbox[1] <= bbox[0]:
             raise IndexError(f"{uid}: empty lobe segmentation (the reference fails in find_objects here)")
         crop = grow_bbox(bbox, scan.shape, spacing, self.crop_border)
         image, lung, ess = ops.lung_crop(scan_d, lobe_d, crop)
-        return {
+        sample = {
             "image": image,
             "lung_mask": lung.view(torch.bool),
             "ess_mask": ess.view(torch.bool),
@@ -76,6 +96,10 @@ class SubtypingInference(torch.utils.data.Dataset):
             "original_size": np.asarray(scan.shape),
             "uid": uid,
         }
+        if self.lobe_labels:
+            (z0, z1), (y0, y1), (x0, x1) = crop
+            sample["lobe_labels"] = lobe_d[z0:z1, y0:y1, x0:x1].contiguous()
+        return sample
 
     def load_raw(self, index):
         """The file half of `get_data` (dataset.py:57-65): read CT + lobes.  Host only and thread-safe, so the

@@ -65,6 +65,13 @@ def _as_u8(mask):
     return (mask != 0).to(torch.uint8)
 
 
+def _lobe_outputs(cle, pse, ess, labels):
+    """The per-label keys of predict_step: voxel counts and both lesion percentages of every label 0..255, each
+    divided by that label's own voxel count (never the batch-wide denominator of quirk Q1)."""
+    pct, voxels = ops.lobe_scores(cle, pse, ess, labels.contiguous())
+    return {"lobe_voxels": voxels, "cle_lobe_percentages": pct[0], "pse_lobe_percentages": pct[1]}
+
+
 class SubtypeDataModule(_DataModuleBase):
     """models.py:36-96 (prediction part): builds `SubtypingInference` with the inference transform."""
 
@@ -83,7 +90,7 @@ class SubtypeDataModule(_DataModuleBase):
     def predict_dataset(self):
         self.datasets[PREDICT_PHASE] = SubtypingInference(
             scan_path=self.args.scan_path, lobe_path=self.args.lobe_path,
-            transforms=self._make_transforms(TEST_PHASE))
+            transforms=self._make_transforms(TEST_PHASE), lobe_labels=bool(getattr(self.args, "lobe_scores", False)))
         return self.datasets[PREDICT_PHASE]
 
     def predict_dataloader(self, rank=0, world_size=1):
@@ -275,7 +282,7 @@ class ScanRegLightningModule(_ScanModule):
                 dense = eng.run_network()
             cle, pse, pct = ops.dram_upsample_mask(dense[0], dense[1], ess, lungs, (D, H, W),
                                                    per_sample_denominator=self.per_sample_percentage)
-            return {
+            out = {
                 "cle_dense_outs": cle,
                 "pse_dense_outs": pse,
                 "cle_precentages": pct[0],
@@ -284,15 +291,20 @@ class ScanRegLightningModule(_ScanModule):
                 "original_size": batch.get("original_size"),
                 "uids": batch.get("uid"),
             }
+            if "lobe_labels" in batch:
+                out.update(_lobe_outputs(cle, pse, ess, self._to_device(batch["lobe_labels"])))
+            return out
 
-    def predict_step_from_hu(self, hu, lung_mask, ess_mask, fuse_window=None):
+    def predict_step_from_hu(self, hu, lung_mask, ess_mask, fuse_window=None, lobe_labels=None):
         """The device-resident hot path of SURVEY §8d: int16 HU volumes already at network size [B,D,H,W] -> K8
         window + standardise (per volume) -> network -> dRAM.  `fuse_window=True`: K8 is its statistics pass plus an
         851-entry table per volume, and the stem convolution clamps and gathers while it loads the int16 volume (the
         same values bit for bit; the fp32 image is never written).  `fuse_window=False`: K8 writes the fp32 image first
         (what predict_step receives from the transforms).  Default (None): env DRAM_B200_FUSE_WINDOW, else False — the
         stem kernel is bound by its producers' instruction issue, and the table gathers cost it more (0.38 against
-        0.23 ms per 256^3 volume, profiles/aux_metrics_r2b.csv) than K8's apply pass saves (0.03 ms).  Returns the same dict as predict_step (without the bookkeeping keys)."""
+        0.23 ms per 256^3 volume, profiles/aux_metrics_r2b.csv) than K8's apply pass saves (0.03 ms).  Returns the same dict as predict_step (without the bookkeeping keys).
+        `lobe_labels`: optional uint8 [B,D,H,W] label volumes; adds the per-label keys predict_step adds for a batch
+        that carries them."""
         with torch.no_grad():
             if not hu.is_cuda or hu.dtype != torch.int16:
                 raise RuntimeError("predict_step_from_hu: expected an int16 CUDA tensor [B,D,H,W]")
@@ -312,8 +324,11 @@ class ScanRegLightningModule(_ScanModule):
             lungs, ess = _as_u8(lung_mask), _as_u8(ess_mask)
             cle, pse, pct = ops.dram_upsample_mask(dense[0], dense[1], ess, lungs, (D, H, W),
                                                    per_sample_denominator=self.per_sample_percentage)
-            return {"cle_dense_outs": cle, "pse_dense_outs": pse, "cle_precentages": pct[0],
-                    "pse_precentages": pct[1]}
+            out = {"cle_dense_outs": cle, "pse_dense_outs": pse, "cle_precentages": pct[0],
+                   "pse_precentages": pct[1]}
+            if lobe_labels is not None:
+                out.update(_lobe_outputs(cle, pse, ess, lobe_labels))
+            return out
 
     def _ratio_to_label(self, ratios, ratio_mapping):
         labels = [ratio_to_label(r.item(), ratio_mapping) for r in ratios]

@@ -5,7 +5,7 @@ raw device pointers plus the current CUDA stream to libdram_b200.so and returns 
 The stateless kernel families are registered as `torch.library.custom_op`s in the `dram_b200::`
 namespace by `custom_ops.py` (imported at the bottom of this module): `torch.ops.dram_b200.conv3d`,
 `.stem_conv7`, `.maxpool3d`, `.upsample2x`, `.masked_pool`, `.dram_upsample_mask`, `.window_standardize`,
-`.resize_image`, `.resize_mask`, `.heatmap_u8`, each with a fake (shape-only) implementation.  The
+`.resize_image`, `.resize_mask`, `.heatmap_u8`, `.lobe_scores`, each with a fake (shape-only) implementation.  The
 functions below are what those ops call; the engine calls them (and its frozen `Conv3dPlan`s) directly
 and replays the whole sequence as one CUDA graph.
 
@@ -515,6 +515,41 @@ def dram_upsample_mask(dense0, dense1, ess, lungs, size, per_sample_denominator=
     return out0, out1, pct
 
 
+LOBE_LABELS = 256
+
+
+def lobe_scores(cle, pse, ess, labels, out=None):
+    """K7l: lesion percentages per label.  cle, pse fp32 [B,1,D,H,W] (the dRAM maps of K7); ess bool or uint8 and
+    labels uint8, both [B,D,H,W].  Returns (pct fp32 [2, B, 256], voxels int64 [B, 256]): voxels[b, k] counts the
+    voxels labelled k; pct[m, b, k] is the sum of map m over the ess voxels labelled k divided by voxels[b, k] (NaN
+    where that is 0).  `out`: optional preallocated (pct, voxels)."""
+    lib = _capi.load()
+    _need(cle, torch.float32, "lobe_scores cle", 5)
+    _need(pse, torch.float32, "lobe_scores pse", 5)
+    if isinstance(ess, torch.Tensor) and ess.dtype == torch.bool:
+        ess = ess.view(torch.uint8)
+    _need(ess, torch.uint8, "lobe_scores ess", 4)
+    _need(labels, torch.uint8, "lobe_scores labels", 4)
+    B, D, H, W = labels.shape
+    if tuple(cle.shape) != (B, 1, D, H, W) or tuple(pse.shape) != (B, 1, D, H, W) or tuple(ess.shape) != (B, D, H, W):
+        raise ValueError(f"lobe_scores: maps {tuple(cle.shape)} / {tuple(pse.shape)} and ess {tuple(ess.shape)} must "
+                         f"match labels {tuple(labels.shape)}")
+    if out is None:
+        pct = torch.empty((2, B, LOBE_LABELS), dtype=torch.float32, device=labels.device)
+        voxels = torch.empty((B, LOBE_LABELS), dtype=torch.int64, device=labels.device)
+    else:
+        pct, voxels = out
+        _need(pct, torch.float32, "lobe_scores out pct", 3)
+        _need(voxels, torch.int64, "lobe_scores out voxels", 2)
+        if tuple(pct.shape) != (2, B, LOBE_LABELS) or tuple(voxels.shape) != (B, LOBE_LABELS):
+            raise ValueError(f"lobe_scores: out must be ([2, {B}, 256], [{B}, 256])")
+    count = D * H * W
+    ws = torch.empty(lib.dram_lobe_workspace_bytes(B, count) // 8, dtype=torch.float64, device=labels.device)
+    check(lib.dram_lobe_sums(_p(cle), _p(pse), _p(ess), _p(labels), _p(pct), _p(voxels), _p(ws), B, count, _stream()),
+          "dram_lobe_sums")
+    return pct, voxels
+
+
 def window_standardize(hu, lo=-1150.0, hi=-300.0, out=None, batched=False):
     """K8: int16 HU -> fp32 standardised window; returns (out, stats).  One volume of any shape (stats fp32 [2]),
     or with `batched` a stack [N, ...] of volumes with per-volume statistics (stats fp32 [N, 2]) in three launches."""
@@ -582,6 +617,22 @@ def resize_mask(x, size):
     out = torch.empty((D2, H2, W2), dtype=torch.uint8, device=x.device)
     check(_capi.load().dram_resize_mask(_p(x), _p(out), _p(idx), D, H, W, D2, H2, W2, _stream()),
           "dram_resize_mask")
+    return out
+
+
+def resize_labels(x, size, out=None):
+    """uint8 label volume [D,H,W] -> `size`: the voxel `resize_mask` picks, its value kept (not cast to 0/1)."""
+    _need(x, torch.uint8, "resize_labels x", 3)
+    D, H, W = x.shape
+    D2, H2, W2 = size
+    idx = slice_index(D, D2, x.device)
+    if out is None:
+        out = torch.empty((D2, H2, W2), dtype=torch.uint8, device=x.device)
+    _need(out, torch.uint8, "resize_labels out", 3)
+    if tuple(out.shape) != (D2, H2, W2):
+        raise ValueError(f"resize_labels: out shape {tuple(out.shape)} != {(D2, H2, W2)}")
+    check(_capi.load().dram_resize_labels(_p(x), _p(out), _p(idx), D, H, W, D2, H2, W2, _stream()),
+          "dram_resize_labels")
     return out
 
 

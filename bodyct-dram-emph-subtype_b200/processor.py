@@ -2,6 +2,7 @@
 
     python processor.py --scan_path DIR --lobe_path DIR --output_path DIR [--ngpus N]
                         [--model_arch med3ddram] [--batch_size 2] [--target_size 128,224,288] [--workers 0]
+                        [--lobe_scores]
 
 Outputs (same names, including the reference's `araseptal-` typo, processor.py:77):
     <out>/images/centrilobular-emphysema-heatmap/<uid>.mha   uint8
@@ -13,6 +14,11 @@ here for --ngpus > 1, each takes the DistributedSampler(shuffle=False) shard of 
 rank 0 merges the per-rank records (the reference lets every rank overwrite results.json, Q8);
 classification architectures (med3d*) are routed to ScanCLSLightningModule and emit argmax classes
 (the reference crashes on them, Q4); --target_size is parseable (Q7); unknown Trainer flags are ignored.
+
+`--lobe_scores` (not in the reference; *dram architectures only) adds to every results.json record
+    "lobe_metrics": {"<label>": {"cle_lesion_percentage": "x.xxx", "pse_lesion_percentage": "y.yyy"}, ...}
+for each label >= 1 of the lobe segmentation that has voxels in the network's grid: the lesion fraction of that
+lobe, in the unit of `*_lesion_percentage_per_lung`.
 """
 import json
 import logging
@@ -65,7 +71,17 @@ def build_parser():
     p.add_argument("--allow_random_init", action="store_true",
                    help="tests/benchmarks only: run with random-init weights when the checkpoint is missing or a Git-LFS "
                         "pointer (recorded in every result's error_messages); without it that is a fatal error")
+    p.add_argument("--lobe_scores", action="store_true",
+                   help="also report CLE and PSE lesion percentages per lobe label (lobe_metrics in results.json); "
+                        "*dram architectures only")
     return p
+
+
+def check_args(args):
+    """Refuses option combinations that cannot run, before any GPU work."""
+    if args.lobe_scores and "dram" not in args.model_arch:
+        raise ValueError(f"--lobe_scores needs a *dram (regression) architecture; {args.model_arch} is a "
+                         "classification architecture without dRAM maps")
 
 
 class CheckpointError(RuntimeError):
@@ -109,12 +125,24 @@ def load_checkpoint(module, path, allow_random_init=False):
     return True
 
 
+def lobe_metrics(voxels, cle_pct, pse_pct):
+    """The `lobe_metrics` field of one record from predict_step's per-label outputs of one sample (voxels [256],
+    percentages [256]): labels >= 1 that have voxels, percentages formatted like the whole-lung ones."""
+    voxels, cle_pct, pse_pct = (torch.as_tensor(v).cpu().tolist() for v in (voxels, cle_pct, pse_pct))
+    return {str(k): {"cle_lesion_percentage": "{:.3f}".format(cle_pct[k]),
+                     "pse_lesion_percentage": "{:.3f}".format(pse_pct[k])}
+            for k in range(1, len(voxels)) if voxels[k] > 0}
+
+
 def postprocess_reg(pred, data_module, out_cle, out_pse, writer=None):
     """processor.py:111-158 for one batch of predictions; returns the result records.  `writer`: a
     `mha_io.BackgroundWriter` that takes the file writes off this thread (`--workers N`)."""
     records = []
     meta_cache = data_module.datasets[RunningStage.PREDICTING].scan_meta_cache
     B = pred["cle_dense_outs"].shape[0]
+    lobes = None
+    if "lobe_voxels" in pred:
+        lobes = [pred[k].cpu() for k in ("lobe_voxels", "cle_lobe_percentages", "pse_lobe_percentages")]
     for b in range(B):
         crop = pred["crop_slices"][b]
         orig = tuple(int(v) for v in pred["original_size"][b])
@@ -130,7 +158,10 @@ def postprocess_reg(pred, data_module, out_cle, out_pse, writer=None):
             "pse_severity_score": "{:d}".format(ratio_to_label(pse_pct, PSE_RATIO_MAP)),
             "pse_lesion_percentage_per_lung": "{:.3f}".format(pse_pct),
         }
-        records.append({"entity": uid, "metrics": metrics, "error_messages": []})
+        record = {"entity": uid, "metrics": metrics, "error_messages": []}
+        if lobes is not None:
+            record["lobe_metrics"] = lobe_metrics(lobes[0][b], lobes[1][b], lobes[2][b])
+        records.append(record)
         meta = meta_cache[uid]
         kw = dict(type=np.uint8, origin=meta["origin"][::-1], spacing=meta["spacing"][::-1],
                   direction=np.asarray(meta["direction"]).reshape(3, 3)[::-1].flatten().tolist())
@@ -214,6 +245,7 @@ def write_results(args, records):
 
 def run_testing_job(argv=None):
     args, _ignored_trainer_flags = build_parser().parse_known_args(argv)
+    check_args(args)
     Path(args.output_path).mkdir(parents=True, exist_ok=True)
     rank = int(os.environ.get("DRAM_B200_RANK", "-1"))
     if rank >= 0:  # worker of a multi-GPU job

@@ -2,7 +2,8 @@
 -> 0,1) -> Standardize -> Interpolate(target_size, align_corners=True, only_in_plane=True)) as two GPU
 kernels per image (K8 window+standardise, K8b in-plane bilinear + slice pick) and one per mask (K8b
 legacy-nearest + slice pick).  Dispatch is by key substring exactly like base.py:119-133: keys containing
-"image" take the image path, keys containing "mask" the mask path, everything else passes through.
+"image" take the image path, keys containing "mask" the mask path, everything else passes through.  One key is
+matched exactly before that: `lobe_labels` (not in the reference) takes the mask path with the label values kept.
 """
 import numpy as np
 import torch
@@ -38,11 +39,18 @@ class InferenceTransform:
         t = t.to(self._dev(), non_blocking=True).contiguous()
         return ops.resize_mask(t, self.target_size).view(torch.bool)
 
+    def apply_to_labels(self, data):
+        """uint8 lobe labels: the mask path with the label values kept."""
+        t = torch.as_tensor(data).to(self._dev(), non_blocking=True).contiguous()
+        return ops.resize_labels(t, self.target_size)
+
     def __call__(self, sample):
         out = {}
         for key, val in sample.items():
             is_array = isinstance(val, (np.ndarray, torch.Tensor))
-            if is_array and "image" in key:
+            if is_array and key == "lobe_labels":
+                out[key] = self.apply_to_labels(val)
+            elif is_array and "image" in key:
                 if key == "original_image" and not self.keep_original_image:
                     continue  # never read by predict_step / the processor; skipped unless asked for
                 out[key] = self.apply_to_image(val)

@@ -267,6 +267,23 @@ int dram_dram_upsample_mask(const float *dense0, const float *dense1, const uint
                             int32_t D, int32_t H, int32_t W, int32_t per_sample_denominator,
                             void *stream);
 
+/* ---- K7l: lesion percentages per label (per lobe) of both dRAM maps ----- */
+/*
+ * Not in the reference (it reports whole-lung numbers only).  map0/map1: fp32 [n][count] (the K7 outputs
+ * [n][1][D][H][W]); ess, labels: uint8 [n][count] (labels: lobe labels resized like the masks).
+ *   voxels[b][k]  int64 [n][256] = #{v : labels[b][v] == k}                                (exact)
+ *   pct[m][b][k]  fp32 [2][n][256] = (float)S / (float)voxels[b][k],
+ *                 S = sum over {v : labels[b][v] == k and ess[b][v] != 0} of map_m[b][v] in fp64
+ *                 (the conversion of K7's percentages; NaN where voxels[b][k] == 0)
+ * The denominator is always the sample's own label volume.  Bit-reproducible: per-CTA partials and a
+ * fixed-order finish, no floating-point atomics.  Map values are read only where ess is set.  ess and
+ * labels that start on a 16-byte boundary with count % 16 == 0 take 16-byte loads, anything else a byte
+ * path.  workspace: dram_lobe_workspace_bytes(n, count) bytes, 8-byte aligned; count < 2^31.
+ */
+size_t dram_lobe_workspace_bytes(int32_t n, int64_t count);
+int dram_lobe_sums(const float *map0, const float *map1, const uint8_t *ess, const uint8_t *labels, float *pct,
+                   int64_t *voxels, void *workspace, int32_t n, int64_t count, void *stream);
+
 /* ---- K8: HU window + standardise (functional.py:13-26,                   */
 /*          intensity_transforms.py:104-114; wired at models.py:60-61) ---- */
 /*
@@ -300,11 +317,15 @@ int dram_window_lut(const int16_t *hu, float *lut, float *stats_out, void *works
  * Image: in-plane bilinear (align_corners=True) to (H2,W2) then slice pick
  * d_idx[k] (the caller builds d_idx with torch.linspace(0,D-1,D2).long(),
  * spatial_transforms.py:66).  Mask: in-plane legacy nearest + same slice pick.
+ * Labels: the voxel the mask rule picks, its value kept instead of cast to 0/1 (lobe labels; not in
+ * the reference), so (labels_out > 0) equals the mask resize of (labels > 0) bit for bit.
  */
 int dram_resize_image(const float *x, float *out, const int32_t *d_idx, int32_t D, int32_t H,
                       int32_t W, int32_t D2, int32_t H2, int32_t W2, void *stream);
 int dram_resize_mask(const uint8_t *x, uint8_t *out, const int32_t *d_idx, int32_t D, int32_t H,
                      int32_t W, int32_t D2, int32_t H2, int32_t W2, void *stream);
+int dram_resize_labels(const uint8_t *x, uint8_t *out, const int32_t *d_idx, int32_t D, int32_t H,
+                       int32_t W, int32_t D2, int32_t H2, int32_t W2, void *stream);
 
 /* ---- f1: device pre-steps of SubtypingInference.get_data (dataset.py:66-80) ---- */
 /*
