@@ -91,6 +91,8 @@ SIGNATURES = {
     "dram_mask_bbox": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp]),
     "dram_lung_crop_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "dram_lung_crop": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "dram_label_counts": (C.c_int, [_vp, _i64, _vp, _vp]),
+    "dram_label_hu_hist": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp]),
     "dram_heatmap_u8": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "dram_conv3d_wgrad_workspace_bytes": (_i64, [C.POINTER(ConvDesc)]),
     "dram_conv3d_wgrad_plan_create": (C.c_int, [C.POINTER(ConvDesc), _vp, _vp, _vp, _i32, _i32, _vp, _i64, C.POINTER(_vp)]),

@@ -9,6 +9,8 @@
 //                       to uint8 — one pass over the output volume, only uint8 leaves the GPU.
 #include <math.h>
 
+#include <atomic>
+
 #include "common.h"
 
 namespace dram {
@@ -260,6 +262,181 @@ heatmap_u8_kernel(const float *__restrict__ map, uint8_t *__restrict__ out, int 
   }
 }
 
+// ---------------------------------------------------------------------------------------
+// Densitometry on the full-resolution grid: voxels per label, and per-slot HU histograms + exact HU sums.
+// A thread takes DENS_VECS 16-voxel vectors per trip (grid-stride).  Runs of equal keys in the order a thread
+// visits its voxels (label; or slot and bin) are folded into one shared atomic, and a run is carried across
+// trips, so a thread that sees only background does one atomic in all.  Each CTA adds its nonzero shared
+// counters into the int64 outputs with integer atomics: exact, whatever the order.
+// ---------------------------------------------------------------------------------------
+static constexpr int DENS_THREADS = 512;
+static constexpr int DENS_VECS = 4;
+static constexpr int HIST_VECS = 2;
+static constexpr int DENS_LABELS = 256;
+static constexpr int HU_BINS = 2048;
+static constexpr int HU_LO = -1024;
+static constexpr int HU_SLOTS = 16;
+static constexpr unsigned NO_SLOT = 0xFFu;
+
+struct SlotTable {
+  uint8_t slot[DENS_LABELS];
+};
+
+// 16 labels of vector v as four little-endian words; zeros past the end of the volume.  nv: voxels in the vector.
+template <bool VEC>
+__device__ __forceinline__ int load_labels16(const uint8_t *__restrict__ lb, int64_t v, int64_t count, uint32_t (&w)[4]) {
+  const int64_t o = v * 16, left = count - o;
+  const int nv = left <= 0 ? 0 : (left >= 16 ? 16 : (int)left);
+  if (VEC && nv == 16) {
+    const uint4 q = __ldg(reinterpret_cast<const uint4 *>(lb + o));
+    w[0] = q.x; w[1] = q.y; w[2] = q.z; w[3] = q.w;
+  } else {
+    w[0] = w[1] = w[2] = w[3] = 0;
+#pragma unroll
+    for (int k = 0; k < 16; ++k)
+      if (k < nv) w[k >> 2] |= (uint32_t)__ldg(lb + o + k) << (8 * (k & 3));
+  }
+  return nv;
+}
+
+__device__ __forceinline__ unsigned byte16(const uint32_t (&w)[4], int k) { return (w[k >> 2] >> (8 * (k & 3))) & 0xffu; }
+
+template <bool VEC>
+__global__ void __launch_bounds__(DENS_THREADS)
+label_counts_kernel(const uint8_t *__restrict__ labels, int64_t count, unsigned long long *__restrict__ counts) {
+  __shared__ uint32_t cnt[DENS_LABELS];
+  for (int i = threadIdx.x; i < DENS_LABELS; i += DENS_THREADS) cnt[i] = 0;
+  __syncthreads();
+  const int64_t vecs = (count + 15) / 16;
+  const int64_t stride = (int64_t)gridDim.x * DENS_THREADS * DENS_VECS;
+  unsigned cur = 0, run = 0;
+  for (int64_t v0 = (int64_t)blockIdx.x * DENS_THREADS * DENS_VECS + threadIdx.x; v0 < vecs; v0 += stride) {
+    uint32_t w[DENS_VECS][4];
+    int nv[DENS_VECS];
+#pragma unroll
+    for (int j = 0; j < DENS_VECS; ++j) nv[j] = load_labels16<VEC>(labels, v0 + j * DENS_THREADS, count, w[j]);
+#pragma unroll
+    for (int j = 0; j < DENS_VECS; ++j) {
+      const uint32_t rep = (w[j][0] & 0xffu) * 0x01010101u;
+      if (nv[j] == 16 && w[j][0] == rep && w[j][1] == rep && w[j][2] == rep && w[j][3] == rep) {  // one label
+        const unsigned lab = rep & 0xffu;
+        if (lab != cur) {
+          if (run) atomicAdd(&cnt[cur], run);
+          cur = lab;
+          run = 0;
+        }
+        run += 16;
+        continue;
+      }
+#pragma unroll
+      for (int k = 0; k < 16; ++k) {
+        if (k >= nv[j]) break;
+        const unsigned lab = byte16(w[j], k);
+        if (lab != cur) {
+          if (run) atomicAdd(&cnt[cur], run);
+          cur = lab;
+          run = 0;
+        }
+        ++run;
+      }
+    }
+  }
+  if (run) atomicAdd(&cnt[cur], run);
+  __syncthreads();
+  for (int i = threadIdx.x; i < DENS_LABELS; i += DENS_THREADS)
+    if (cnt[i]) atomicAdd(&counts[i], (unsigned long long)cnt[i]);
+}
+
+// Dynamic shared memory: nslots x 2048 uint32 bins (up to 128 KB).  The vector path keeps to 64 registers, so that two
+// CTAs fit an SM whenever their bins do (the byte path, for unaligned views only, would spill there).
+template <bool VEC>
+__global__ void __launch_bounds__(DENS_THREADS, VEC ? 2 : 1)
+label_hu_hist_kernel(const int16_t *__restrict__ scan, const uint8_t *__restrict__ labels, int64_t count,
+                     const SlotTable table, int nslots, unsigned long long *__restrict__ hist,
+                     unsigned long long *__restrict__ hu_sum) {
+  extern __shared__ uint4 bins_raw[];
+  uint32_t *bins = reinterpret_cast<uint32_t *>(bins_raw);
+  __shared__ uint8_t slot_of[DENS_LABELS];
+  __shared__ unsigned long long ssum[HU_SLOTS];
+  const int nbins = nslots * HU_BINS;
+  for (int i = threadIdx.x; i < nbins / 4; i += DENS_THREADS) bins_raw[i] = make_uint4(0, 0, 0, 0);
+  for (int i = threadIdx.x; i < DENS_LABELS; i += DENS_THREADS) slot_of[i] = table.slot[i];
+  if (threadIdx.x < HU_SLOTS) ssum[threadIdx.x] = 0ull;
+  __syncthreads();
+  const bool zero_tracked = table.slot[0] != NO_SLOT;  // label 0 fills most of a chest scan: usually untracked
+  const int64_t vecs = (count + 15) / 16;
+  const int64_t stride = (int64_t)gridDim.x * DENS_THREADS * HIST_VECS;
+  unsigned key = 0, krun = 0;        // run of one (slot, bin): bins[key] += krun
+  unsigned scur = NO_SLOT;           // run of one slot: ssum[scur] += srun
+  long long srun = 0;
+  for (int64_t v0 = (int64_t)blockIdx.x * DENS_THREADS * HIST_VECS + threadIdx.x; v0 < vecs; v0 += stride) {
+    uint32_t sw[HIST_VECS][4];       // labels, then their slots (NO_SLOT past the end)
+    int nv[HIST_VECS];
+    bool tracked[HIST_VECS];
+#pragma unroll
+    for (int j = 0; j < HIST_VECS; ++j) nv[j] = load_labels16<VEC>(labels, v0 + j * DENS_THREADS, count, sw[j]);
+#pragma unroll
+    for (int j = 0; j < HIST_VECS; ++j) {
+      tracked[j] = false;
+      if (nv[j] == 0 || (!zero_tracked && (sw[j][0] | sw[j][1] | sw[j][2] | sw[j][3]) == 0u)) continue;
+      uint32_t s4[4] = {0, 0, 0, 0};
+#pragma unroll
+      for (int k = 0; k < 16; ++k) {
+        const unsigned s = k < nv[j] ? (unsigned)slot_of[byte16(sw[j], k)] : NO_SLOT;
+        tracked[j] |= s != NO_SLOT;
+        s4[k >> 2] |= s << (8 * (k & 3));
+      }
+#pragma unroll
+      for (int q = 0; q < 4; ++q) sw[j][q] = s4[q];
+    }
+    // the HU of every whole tracked vector of the trip, loaded before any is used (the byte path loads per voxel)
+    uint4 hu[HIST_VECS][2];
+#pragma unroll
+    for (int j = 0; j < HIST_VECS; ++j) {
+      hu[j][0] = hu[j][1] = make_uint4(0, 0, 0, 0);
+      if (VEC && tracked[j] && nv[j] == 16) {
+        const uint4 *p = reinterpret_cast<const uint4 *>(scan + (v0 + j * DENS_THREADS) * 16);
+        hu[j][0] = __ldg(p);
+        hu[j][1] = __ldg(p + 1);
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < HIST_VECS; ++j) {
+      if (!tracked[j]) continue;
+      const bool whole = VEC && nv[j] == 16;
+      const int16_t *sp = scan + (v0 + j * DENS_THREADS) * 16;
+      const uint32_t hw[8] = {hu[j][0].x, hu[j][0].y, hu[j][0].z, hu[j][0].w,
+                              hu[j][1].x, hu[j][1].y, hu[j][1].z, hu[j][1].w};
+#pragma unroll
+      for (int k = 0; k < 16; ++k) {
+        const unsigned s = byte16(sw[j], k);
+        if (s == NO_SLOT) continue;  // also every voxel past the end of the volume
+        const int h = whole ? (int)(short)(uint16_t)(hw[k >> 1] >> (16 * (k & 1))) : (int)__ldg(sp + k);
+        const unsigned b = (unsigned)(min(max(h, HU_LO), HU_LO + HU_BINS - 1) - HU_LO);
+        const unsigned kk = s * HU_BINS + b;
+        if (kk != key) {
+          if (krun) atomicAdd(&bins[key], krun);
+          key = kk;
+          krun = 0;
+        }
+        ++krun;
+        if (s != scur) {
+          if (scur != NO_SLOT) atomicAdd(&ssum[scur], (unsigned long long)srun);
+          scur = s;
+          srun = 0;
+        }
+        srun += h;
+      }
+    }
+  }
+  if (krun) atomicAdd(&bins[key], krun);
+  if (scur != NO_SLOT) atomicAdd(&ssum[scur], (unsigned long long)srun);
+  __syncthreads();
+  for (int i = threadIdx.x; i < nbins; i += DENS_THREADS)
+    if (bins[i]) atomicAdd(&hist[i], (unsigned long long)bins[i]);
+  if (threadIdx.x < nslots && ssum[threadIdx.x]) atomicAdd(&hu_sum[threadIdx.x], ssum[threadIdx.x]);
+}
+
 }  // namespace dram
 
 using namespace dram;
@@ -326,4 +503,87 @@ extern "C" int dram_heatmap_u8(const float *map, int32_t d, int32_t h, int32_t w
       map, out, d, h, w, OD, OH, OW, z0, y0, x0, cd, ch, cw, ac_scale(d, cd), ac_scale(h, ch), ac_scale(w, cw));
   DRAM_CHECK_LAUNCH("heatmap_u8_kernel");
   return DRAM_OK;
+}
+
+// Grid of the densitometry passes: enough CTAs to fill the device, no more than there are trips.
+static int dens_grid(int64_t count, int vecs_per_trip, int ctas_per_sm) {
+  const int64_t trips = ceil_div64(ceil_div64(count, 16), (int64_t)DENS_THREADS * vecs_per_trip);
+  const int64_t cap = (int64_t)sm_count() * (ctas_per_sm < 1 ? 1 : ctas_per_sm);
+  return (int)(trips < 1 ? 1 : (trips < cap ? trips : cap));
+}
+
+extern "C" int dram_label_counts(const uint8_t *labels, int64_t count, int64_t *counts, void *stream) {
+  DRAM_REQUIRE(labels && counts, "dram_label_counts: null pointer");
+  DRAM_REQUIRE(count >= 0 && count < 0x7fffffffLL, "dram_label_counts: count %lld outside 0 .. 2^31-1",
+               (long long)count);
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = check_cuda(cudaMemsetAsync(counts, 0, DENS_LABELS * sizeof(int64_t), st), "dram_label_counts: zeroing");
+  if (rc != DRAM_OK || count == 0) return rc;
+  unsigned long long *out = reinterpret_cast<unsigned long long *>(counts);
+  if ((uintptr_t)labels % 16 == 0)
+    label_counts_kernel<true><<<dens_grid(count, DENS_VECS, 4), DENS_THREADS, 0, st>>>(labels, count, out);
+  else
+    label_counts_kernel<false><<<dens_grid(count, DENS_VECS, 4), DENS_THREADS, 0, st>>>(labels, count, out);
+  DRAM_CHECK_LAUNCH("label_counts_kernel");
+  return DRAM_OK;
+}
+
+// CTAs of the histogram kernel per SM for `nslots` slots.  The shared-memory attribute and the occupancy query run on the
+// first call per device and slot count only, so that later calls (e.g. under stream capture) make no such API call.
+template <bool VEC>
+static int hu_hist_ctas_per_sm(int nslots, int *per_sm) {
+  static std::atomic<int> known[64][HU_SLOTS + 1];
+  int dev = 0;
+  int rc = check_cuda(cudaGetDevice(&dev), "dram_label_hu_hist: device");
+  if (rc != DRAM_OK) return rc;
+  if (dev >= 0 && dev < 64 && (*per_sm = known[dev][nslots].load()) > 0) return DRAM_OK;
+  auto kernel = label_hu_hist_kernel<VEC>;
+  rc = check_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       HU_SLOTS * HU_BINS * (int)sizeof(uint32_t)),
+                  "dram_label_hu_hist: shared memory attribute");
+  if (rc != DRAM_OK) return rc;
+  rc = check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, kernel, DENS_THREADS,
+                                                                 (size_t)nslots * HU_BINS * sizeof(uint32_t)),
+                  "dram_label_hu_hist: occupancy");
+  if (rc != DRAM_OK) return rc;
+  if (*per_sm < 1) *per_sm = 1;
+  if (dev >= 0 && dev < 64) known[dev][nslots].store(*per_sm);
+  return DRAM_OK;
+}
+
+template <bool VEC>
+static int launch_hu_hist(const int16_t *scan, const uint8_t *labels, int64_t count, const SlotTable &table,
+                          int nslots, unsigned long long *hist, unsigned long long *hu_sum, cudaStream_t st) {
+  int per_sm = 0;
+  int rc = hu_hist_ctas_per_sm<VEC>(nslots, &per_sm);
+  if (rc != DRAM_OK) return rc;
+  label_hu_hist_kernel<VEC><<<dens_grid(count, HIST_VECS, per_sm), DENS_THREADS,
+                              (size_t)nslots * HU_BINS * sizeof(uint32_t), st>>>(scan, labels, count, table, nslots,
+                                                                                 hist, hu_sum);
+  DRAM_CHECK_LAUNCH("label_hu_hist_kernel");
+  return DRAM_OK;
+}
+
+extern "C" int dram_label_hu_hist(const int16_t *scan, const uint8_t *labels, int64_t count,
+                                  const uint8_t *slot_of_label, int32_t nslots, int64_t *hist, int64_t *hu_sum,
+                                  void *stream) {
+  DRAM_REQUIRE(scan && labels && slot_of_label && hist && hu_sum, "dram_label_hu_hist: null pointer");
+  DRAM_REQUIRE(nslots >= 1 && nslots <= HU_SLOTS, "dram_label_hu_hist: nslots %d outside 1..%d", nslots, HU_SLOTS);
+  DRAM_REQUIRE(count >= 0 && count < 0x7fffffffLL, "dram_label_hu_hist: count %lld outside 0 .. 2^31-1",
+               (long long)count);
+  SlotTable table;
+  for (int k = 0; k < DENS_LABELS; ++k) {
+    DRAM_REQUIRE(slot_of_label[k] < nslots || slot_of_label[k] == NO_SLOT,
+                 "dram_label_hu_hist: label %d goes to slot %d of %d", k, (int)slot_of_label[k], nslots);
+    table.slot[k] = slot_of_label[k];
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = check_cuda(cudaMemsetAsync(hist, 0, (size_t)nslots * HU_BINS * sizeof(int64_t), st),
+                      "dram_label_hu_hist: zeroing");
+  if (rc == DRAM_OK) rc = check_cuda(cudaMemsetAsync(hu_sum, 0, (size_t)nslots * sizeof(int64_t), st),
+                                     "dram_label_hu_hist: zeroing");
+  if (rc != DRAM_OK || count == 0) return rc;
+  unsigned long long *h = reinterpret_cast<unsigned long long *>(hist), *s = reinterpret_cast<unsigned long long *>(hu_sum);
+  if (((uintptr_t)scan | (uintptr_t)labels) % 16 == 0) return launch_hu_hist<true>(scan, labels, count, table, nslots, h, s, st);
+  return launch_hu_hist<false>(scan, labels, count, table, nslots, h, s, st);
 }

@@ -178,5 +178,31 @@ def _(dram_map, crop, original_size):
     return dram_map.new_empty(tuple(original_size), dtype=torch.uint8)
 
 
+# ------------------------------------------------------------------------------------------------ densitometry
+@custom_op(f"{NS}::label_counts", mutates_args=(), device_types="cuda")
+def label_counts(labels: torch.Tensor) -> torch.Tensor:
+    """Voxels per label of a uint8 label volume: int64 [256]."""
+    return ops.label_counts(labels)
+
+
+@label_counts.register_fake
+def _(labels):
+    return labels.new_empty((ops.LOBE_LABELS,), dtype=torch.int64)
+
+
+@custom_op(f"{NS}::hu_histograms", mutates_args=(), device_types="cuda")
+def hu_histograms(scan: torch.Tensor, labels: torch.Tensor, label_ids: List[int]) -> Tuple[torch.Tensor, torch.Tensor]:
+    """HU histograms (clamped to [-1024, 1023], 2048 bins) and exact HU sums of the voxels of each listed label:
+    (int64 [len(ids), 2048], int64 [len(ids)])."""
+    return ops.hu_histograms(scan, labels, label_ids)
+
+
+@hu_histograms.register_fake
+def _(scan, labels, label_ids):
+    n = len(label_ids)
+    return scan.new_empty((n, ops.HU_BINS), dtype=torch.int64), scan.new_empty((n,), dtype=torch.int64)
+
+
 REGISTERED = ("conv3d", "stem_conv7", "maxpool3d", "upsample2x", "masked_pool", "dram_upsample_mask",
-              "window_standardize", "resize_image", "resize_mask", "heatmap_u8", "lobe_scores")
+              "window_standardize", "resize_image", "resize_mask", "heatmap_u8", "lobe_scores", "label_counts",
+              "hu_histograms")

@@ -47,17 +47,19 @@ class SubtypingInference(torch.utils.data.Dataset):
     label_to_pse = {0: "absent", 1: "mild", 2: "substantial"}
 
     def __init__(self, scan_path, lobe_path, transforms=None, keep_sorted=True, crop_border=5, device=None,
-                 lobe_labels=False):
+                 lobe_labels=False, densitometry=False):
         """`lobe_labels=True`: every sample also carries `lobe_labels`, the uint8 label volume cropped like the masks
-        (for the per-lobe percentages)."""
+        (for the per-lobe percentages).  `densitometry=True`: the pre-steps also measure the lung and every lobe label
+        on the full-resolution scan (`densitometry.scan_densitometry`) into `densitometry_cache[uid]`."""
         super().__init__()
         self.device = torch.device(device) if device is not None else getattr(transforms, "device", None)
         self.scan_path, self.lobe_path = scan_path, lobe_path
         self.keep_sorted, self.transforms, self.crop_border = keep_sorted, transforms, crop_border
-        self.lobe_labels = lobe_labels
+        self.lobe_labels, self.densitometry = lobe_labels, densitometry
         self.scan_files = sorted(glob.glob(os.path.join(scan_path, "*.mha")))
         self.lobe_files = sorted(glob.glob(os.path.join(lobe_path, "*.mha")))
         self.scan_meta_cache = {}
+        self.densitometry_cache = {}
 
     def __len__(self):
         return len(self.scan_files)
@@ -77,7 +79,7 @@ class SubtypingInference(torch.utils.data.Dataset):
 
         dev = self.device
         scan_d = torch.as_tensor(np.ascontiguousarray(scan)).to(torch.int16).to(dev, non_blocking=True)
-        if self.lobe_labels:  # values kept: lung_crop takes labels > 0 itself
+        if self.lobe_labels or self.densitometry:  # values kept: lung_crop takes labels > 0 itself
             lobe_d = torch.as_tensor(np.ascontiguousarray(labels_as_u8(lobe, uid))).to(dev, non_blocking=True)
         else:
             lobe_d = torch.as_tensor(np.ascontiguousarray(lobe))
@@ -88,6 +90,10 @@ class SubtypingInference(torch.utils.data.Dataset):
             raise IndexError(f"{uid}: empty lobe segmentation (the reference fails in find_objects here)")
         crop = grow_bbox(bbox, scan.shape, spacing, self.crop_border)
         image, lung, ess = ops.lung_crop(scan_d, lobe_d, crop)
+        if self.densitometry:
+            from .densitometry import scan_densitometry
+
+            self.densitometry_cache[uid] = scan_densitometry(scan_d, lobe_d, spacing)
         sample = {
             "image": image,
             "lung_mask": lung.view(torch.bool),

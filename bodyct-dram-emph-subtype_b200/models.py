@@ -90,7 +90,8 @@ class SubtypeDataModule(_DataModuleBase):
     def predict_dataset(self):
         self.datasets[PREDICT_PHASE] = SubtypingInference(
             scan_path=self.args.scan_path, lobe_path=self.args.lobe_path,
-            transforms=self._make_transforms(TEST_PHASE), lobe_labels=bool(getattr(self.args, "lobe_scores", False)))
+            transforms=self._make_transforms(TEST_PHASE), lobe_labels=bool(getattr(self.args, "lobe_scores", False)),
+            densitometry=bool(getattr(self.args, "densitometry", False)))
         return self.datasets[PREDICT_PHASE]
 
     def predict_dataloader(self, rank=0, world_size=1):

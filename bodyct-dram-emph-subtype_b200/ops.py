@@ -5,8 +5,8 @@ raw device pointers plus the current CUDA stream to libdram_b200.so and returns 
 The stateless kernel families are registered as `torch.library.custom_op`s in the `dram_b200::`
 namespace by `custom_ops.py` (imported at the bottom of this module): `torch.ops.dram_b200.conv3d`,
 `.stem_conv7`, `.maxpool3d`, `.upsample2x`, `.masked_pool`, `.dram_upsample_mask`, `.window_standardize`,
-`.resize_image`, `.resize_mask`, `.heatmap_u8`, `.lobe_scores`, each with a fake (shape-only) implementation.  The
-functions below are what those ops call; the engine calls them (and its frozen `Conv3dPlan`s) directly
+`.resize_image`, `.resize_mask`, `.heatmap_u8`, `.lobe_scores`, `.label_counts`, `.hu_histograms`, each with a fake
+(shape-only) implementation.  The functions below are what those ops call; the engine calls them (and its frozen `Conv3dPlan`s) directly
 and replays the whole sequence as one CUDA graph.
 
 Activations are NDHWC 16-bit tensors of shape [N, D, H, W, C]: torch.bfloat16 or torch.float16
@@ -673,6 +673,43 @@ def lung_crop(scan, lobe, crop, out=None):
     check(lib.dram_lung_crop(_p(scan), _p(lobe), D, H, W, z0, y0, x0, cd, ch, cw, _p(image), _p(lung), _p(ess),
                              _p(ws), _stream()), "dram_lung_crop")
     return image, lung, ess
+
+
+HU_BINS = 2048      # HU histogram bins: bin b holds HU b - 1024 (values clamped to [-1024, 1023])
+HU_SLOTS = 16       # labels per histogram pass
+
+
+def label_counts(labels):
+    """Voxels per label of a uint8 label volume (any shape): int64 [256] on the device, exact."""
+    _need(labels, torch.uint8, "label_counts labels")
+    counts = torch.empty(LOBE_LABELS, dtype=torch.int64, device=labels.device)
+    check(_capi.load().dram_label_counts(_p(labels), labels.numel(), _p(counts), _stream()), "dram_label_counts")
+    return counts
+
+
+def hu_histograms(scan, labels, label_ids):
+    """HU histograms of the voxels of each label in `label_ids` (distinct ints in 0..255): int16 scan and uint8 labels
+    of one shape.  Returns (hist int64 [len(ids), 2048], hu_sum int64 [len(ids)]) on the device: hist[i, b] counts
+    the voxels labelled label_ids[i] whose HU, clamped to [-1024, 1023], is b - 1024; hu_sum[i] is the exact sum of
+    their unclamped HU.  One pass per group of 16 labels; no host synchronisation."""
+    lib = _capi.load()
+    _need(scan, torch.int16, "hu_histograms scan")
+    _need(labels, torch.uint8, "hu_histograms labels")
+    if scan.shape != labels.shape:
+        raise ValueError(f"hu_histograms: scan {tuple(scan.shape)} and labels {tuple(labels.shape)} differ in shape")
+    ids = [int(k) for k in label_ids]
+    if any(not 0 <= k < LOBE_LABELS for k in ids) or len(set(ids)) != len(ids):
+        raise ValueError(f"hu_histograms: label ids must be distinct values in 0..255, got {ids}")
+    hist = torch.empty((len(ids), HU_BINS), dtype=torch.int64, device=scan.device)
+    hu_sum = torch.empty(len(ids), dtype=torch.int64, device=scan.device)
+    for g in range(0, len(ids), HU_SLOTS):
+        group = ids[g:g + HU_SLOTS]
+        table = bytearray(b"\xff" * LOBE_LABELS)
+        for s, k in enumerate(group):
+            table[k] = s
+        check(lib.dram_label_hu_hist(_p(scan), _p(labels), scan.numel(), bytes(table), len(group), _p(hist[g:]),
+                                     _p(hu_sum[g:]), _stream()), "dram_label_hu_hist")
+    return hist, hu_sum
 
 
 def heatmap_u8(dram_map, crop, original_size, out=None):

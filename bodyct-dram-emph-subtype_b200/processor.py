@@ -2,7 +2,7 @@
 
     python processor.py --scan_path DIR --lobe_path DIR --output_path DIR [--ngpus N]
                         [--model_arch med3ddram] [--batch_size 2] [--target_size 128,224,288] [--workers 0]
-                        [--lobe_scores]
+                        [--lobe_scores] [--densitometry]
 
 Outputs (same names, including the reference's `araseptal-` typo, processor.py:77):
     <out>/images/centrilobular-emphysema-heatmap/<uid>.mha   uint8
@@ -19,6 +19,11 @@ classification architectures (med3d*) are routed to ScanCLSLightningModule and e
     "lobe_metrics": {"<label>": {"cle_lesion_percentage": "x.xxx", "pse_lesion_percentage": "y.yyy"}, ...}
 for each label >= 1 of the lobe segmentation that has voxels in the network's grid: the lesion fraction of that
 lobe, in the unit of `*_lesion_percentage_per_lung`.
+
+`--densitometry` (not in the reference; every architecture) adds to every results.json record
+    "densitometry": {"lung": {...}, "lobes": {"<label>": {...}, ...}}
+with "volume_ml", "laa950_percentage", "laa910_percentage", "perc15_hu" and "mean_hu" of the lung (all labels >= 1)
+and of each label >= 1 that has voxels, measured on the full-resolution scan (definitions in densitometry.py).
 """
 import json
 import logging
@@ -41,6 +46,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from . import mha_io, ops  # noqa: E402
+from .densitometry import format_densitometry  # noqa: E402
 from .models import (CLE_RATIO_MAP, PSE_RATIO_MAP, RunningStage, ScanCLSLightningModule,  # noqa: E402
                      ScanRegLightningModule, SubtypeDataModule, ratio_to_label)
 from .utils import load_state_dict_greedy, windowing, write_array_to_mha_itk  # noqa: E402
@@ -74,6 +80,9 @@ def build_parser():
     p.add_argument("--lobe_scores", action="store_true",
                    help="also report CLE and PSE lesion percentages per lobe label (lobe_metrics in results.json); "
                         "*dram architectures only")
+    p.add_argument("--densitometry", action="store_true",
+                   help="also report lung and per-lobe volume, %%LAA-950, %%LAA-910, Perc15 and mean HU of the "
+                        "full-resolution scan (densitometry in results.json); every architecture")
     return p
 
 
@@ -161,6 +170,7 @@ def postprocess_reg(pred, data_module, out_cle, out_pse, writer=None):
         record = {"entity": uid, "metrics": metrics, "error_messages": []}
         if lobes is not None:
             record["lobe_metrics"] = lobe_metrics(lobes[0][b], lobes[1][b], lobes[2][b])
+        add_densitometry(record, data_module)
         records.append(record)
         meta = meta_cache[uid]
         kw = dict(type=np.uint8, origin=meta["origin"][::-1], spacing=meta["spacing"][::-1],
@@ -173,13 +183,23 @@ def postprocess_reg(pred, data_module, out_cle, out_pse, writer=None):
     return records
 
 
-def postprocess_cls(pred):
+def postprocess_cls(pred, data_module=None):
     records = []
     for b, uid in enumerate(pred["uids"]):
         metrics = {"cle_severity_score": "{:d}".format(int(pred["cle_labels"][b])),
                    "pse_severity_score": "{:d}".format(int(pred["pse_labels"][b]))}
-        records.append({"entity": uid, "metrics": metrics, "error_messages": []})
+        record = {"entity": uid, "metrics": metrics, "error_messages": []}
+        if data_module is not None:
+            add_densitometry(record, data_module)
+        records.append(record)
     return records
+
+
+def add_densitometry(record, data_module):
+    """Adds the `densitometry` field to a record when the dataset measured its scan (`--densitometry`)."""
+    ds = data_module.datasets[RunningStage.PREDICTING]
+    if getattr(ds, "densitometry", False):
+        record["densitometry"] = format_densitometry(ds.densitometry_cache[record["entity"]])
 
 
 def run_rank(args, rank, world_size):
@@ -214,7 +234,7 @@ def run_rank(args, rank, world_size):
             if is_reg:
                 records += postprocess_reg(pred, data_module, out_cle, out_pse, writer if workers > 0 else None)
             else:
-                records += postprocess_cls(pred)
+                records += postprocess_cls(pred, data_module)
     if not loaded:
         notes.append(RANDOM_INIT_NOTE)
     for r in records:

@@ -349,6 +349,27 @@ size_t dram_lung_crop_workspace_bytes(int32_t cd, int32_t ch, int32_t cw);
 int dram_lung_crop(const int16_t *scan, const uint8_t *lobe, int32_t D, int32_t H, int32_t W, int32_t z0,
                    int32_t y0, int32_t x0, int32_t cd, int32_t ch, int32_t cw, int16_t *image_c,
                    uint8_t *lung_c, uint8_t *ess_c, void *workspace, void *stream);
+/*
+ * Densitometry on the full-resolution grid (not in the reference): the same device scan and uint8 lobe
+ * labels the two calls above read, count voxels.  Both calls zero their own outputs, keep privatised
+ * per-CTA counters in shared memory and add them into the int64 outputs with integer atomics, so the
+ * result is exact and the same in any order.  Labels that start on a 16-byte boundary take 16-byte loads
+ * (the scan too, for the histograms); other views and the last count % 16 voxels take a byte path.
+ * 0 <= count < 2^31.  No host synchronisation and no host-to-device copy: both are graph-capturable.
+ *
+ * dram_label_counts: counts (device int64 [256])[k] = #{v : labels[v] == k}.
+ */
+int dram_label_counts(const uint8_t *labels, int64_t count, int64_t *counts, void *stream);
+/*
+ * dram_label_hu_hist: HU histograms of up to 16 labels in one pass.  slot_of_label is a HOST array of
+ * 256 bytes (passed to the kernel by value): the slot 0 .. nslots-1 label k goes to, or 0xFF for a label
+ * that is not tracked.  1 <= nslots <= 16.  For every slot s (outputs device int64):
+ *   hist[s][b]  = #{v : slot_of_label[labels[v]] == s and clamp(scan[v], -1024, 1023) == b - 1024}
+ *   hu_sum[s]   = sum of scan[v] (unclamped) over the same voxels
+ * The scan is read only for 16-voxel vectors that hold a tracked label.
+ */
+int dram_label_hu_hist(const int16_t *scan, const uint8_t *labels, int64_t count, const uint8_t *slot_of_label,
+                       int32_t nslots, int64_t *hist, int64_t *hu_sum, void *stream);
 
 /* ---- f2: device post-processing of one scan (processor.py:111-158, utils.py:28-37) ---- */
 /*
