@@ -61,6 +61,9 @@ SIGNATURES = {
     "dram_conv3d_run": (C.c_int, [_vp, _i32, _vp]),
     "dram_conv3d_plan_info": (C.c_int, [_vp, C.POINTER(_i64), _pi32, _pi32, _pi32, _pi32]),
     "dram_conv3d_plan_executed_flops": (C.c_int, [_vp, C.POINTER(_i64)]),
+    "dram_conv3d_worklist_size": (C.c_int, [_vp, _pi32]),
+    "dram_conv3d_worklist": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp]),
+    "dram_conv3d_run_listed": (C.c_int, [_vp, _vp, _vp, _i32, _vp]),
     "dram_stem_expand": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp]),
     "dram_stem_weight_bytes": (_sz, []),
     "dram_stem_conv7": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
@@ -71,6 +74,10 @@ SIGNATURES = {
     "dram_upsample2x_plan_create": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, C.POINTER(_vp)]),
     "dram_upsample2x_plan_destroy": (C.c_int, [_vp]),
     "dram_upsample2x_plan_run": (C.c_int, [_vp, _i32, _vp]),
+    "dram_upsample2x_worklist_size": (C.c_int, [_vp, _pi32]),
+    "dram_upsample2x_worklist": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp]),
+    "dram_upsample2x_plan_run_listed": (C.c_int, [_vp, _vp, _vp, _i32, _vp]),
+    "dram_decoder_support": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "dram_upconv_axis": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i64, _i32, _i32, _i32, _vp]),
     "dram_pool_workspace_bytes": (_sz, [_i32, _i32]),
     "dram_masked_pool": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),

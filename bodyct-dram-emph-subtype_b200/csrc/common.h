@@ -37,6 +37,12 @@ inline int check_cuda(cudaError_t e, const char *what) {
 inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// decoder_mask.cu: the ascending list (and count) of the `total` items of a kernel whose tw x th x td output box, grown
+// by `radius` voxels, meets the support bit mask `bits` [n][d][h][ceil(w/32)] (dram_decoder_support).  Items are
+// numbered with D fastest (d_fastest) or W fastest; `flags` is scratch of `total` bytes.
+int worklist_build(const uint32_t *bits, int n, int d, int h, int w, int tw, int th, int td, int d_fastest, int radius,
+                   uint8_t *flags, int *list, int *count, int total, cudaStream_t st);
+
 // Grid for grid-stride memory-bound kernels: a multiple of the SM count.
 int sm_count();
 inline int stream_grid(int64_t work_items, int threads, int ctas_per_sm = 8) {

@@ -172,19 +172,25 @@ conv3d_slab_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
   tmem_base = __shfl_sync(0xffffffffu, tmem_base, 0);  // provably warp-uniform
 
-  // contiguous, balanced range of work items for this CTA
-  const int item_begin = (int)(((long long)blockIdx.x * p.items_total) / gridDim.x);
-  const int item_end = (int)(((long long)(blockIdx.x + 1) * p.items_total) / gridDim.x);
+  // contiguous, balanced range of work items (positions in the work list, if there is one) for this CTA
+  const int items_total = p.items ? *p.count : p.items_total;
+  const int item_begin = (int)(((long long)blockIdx.x * items_total) / gridDim.x);
+  const int item_end = (int)(((long long)(blockIdx.x + 1) * items_total) / gridDim.x);
+  auto item_at = [&](int i) { return p.items ? __ldg(p.items + i) : i; };
   const bool single_chunk = !UP && p.chunks_total == 1;  // UP layers never reuse planes across items
 
   if (warp == SL_A_WARP) {
     if (lane == 0) {
       unsigned seq_end = 0;
       unsigned lseq = 0;  // UP: running index of low-resolution planes through the LP ring
-      for (int item = item_begin; item < item_end; ++item) {
+      int prev = -1;
+      for (int i = item_begin; i < item_end; ++i) {
+        const int item = item_at(i);
         const SlabItem it = decode_item(p, item, Cfg::GROUP);
+        // two planes of the previous item are reused if it was the previous group of the same column
+        const bool reuse = single_chunk && prev == item - 1 && it.g > 0;
+        prev = item;
         for (int c = 0; c < p.chunks_total; ++c) {
-          const bool reuse = single_chunk && item > item_begin && it.g > 0;
           const unsigned seq_base = seq_end - (reuse ? 2u : 0u);
           seq_end = seq_base + ITEM_PLANES;
           if (UP && c < p.chunks1) {
@@ -228,7 +234,7 @@ conv3d_slab_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int item = item_begin; item < item_end; ++item) {
+      for (int i = item_begin; i < item_end; ++i) {
         for (int c = 0; c < p.chunks_total; ++c) {
           for (int hw = 0; hw < 9; ++hw) {  // one stage = the three kd taps of (kh,kw), kd descending
             mbar_wait(b_empty(stage), phase ^ 1u);
@@ -267,14 +273,18 @@ conv3d_slab_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
       unsigned seq_end = 0;
       int buf = 0;
       uint32_t buf_phase = 0;
-      for (int item = item_begin; item < item_end; ++item) {
+      int prev = -1;
+      for (int i = item_begin; i < item_end; ++i) {
+        const int item = item_at(i);
         const SlabItem it = decode_item(p, item, Cfg::GROUP);
         mbar_wait(tmem_empty(buf), buf_phase ^ 1u);
         tcgen05_fence_after();
         const uint32_t tmem_d0 = tmem_base + (uint32_t)(buf * SL_GROUP * BLOCK_N);
+        // the same rule as the producer's: the next list entry is the next group of this column
+        const bool reuse = single_chunk && prev == item - 1 && it.g > 0;
+        const bool next_reuse = single_chunk && i + 1 < item_end && it.g + 1 < p.groups_d && item_at(i + 1) == item + 1;
+        prev = item;
         for (int c = 0; c < p.chunks_total; ++c) {
-          const bool reuse = single_chunk && item > item_begin && it.g > 0;
-          const bool next_reuse = single_chunk && (item + 1 < item_end) && (it.g + 1 < p.groups_d);
           const unsigned seq_base = seq_end - (reuse ? 2u : 0u);
           seq_end = seq_base + ITEM_PLANES;
           // per-plane constants of this chunk: A descriptor of the slot base, barrier addresses / parities
@@ -404,8 +414,8 @@ conv3d_slab_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
     const int tid = threadIdx.x - UP_WARP0 * 32;
     const int is_f16 = p.epi.is_f16;
     unsigned seq_end = 0, lseq_base = 0;
-    for (int item = item_begin; item < item_end; ++item) {
-      const SlabItem it = decode_item(p, item, Cfg::GROUP);
+    for (int i = item_begin; i < item_end; ++i) {
+      const SlabItem it = decode_item(p, item_at(i), Cfg::GROUP);
       for (int c = 0; c < p.chunks_total; ++c) {
         const unsigned seq_base = seq_end;  // UP layers have more than one chunk: no plane reuse across items
         seq_end = seq_base + ITEM_PLANES;
@@ -492,8 +502,8 @@ conv3d_slab_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
     const int lh = row >> 3;
     int buf = 0;
     uint32_t buf_phase = 0;
-    for (int item = item_begin; item < item_end; ++item) {
-      const SlabItem it = decode_item(p, item, Cfg::GROUP);
+    for (int i = item_begin; i < item_end; ++i) {
+      const SlabItem it = decode_item(p, item_at(i), Cfg::GROUP);
       const int oh = it.h0 + lh, ow = it.w0 + lw;
       // residual rows are loaded one 32-channel group ahead (also across the planes of the item); the first one
       // before the wait for the accumulator
@@ -567,12 +577,21 @@ struct StreamCfg {
 struct StreamSeg {
   int sample, w0, h0, t0, t1;
 };
-__device__ __forceinline__ StreamSeg stream_segment(const SlabParams &p, int step, int step_end) {
+// The segment that starts at position `pos` of the CTA's range [.., pos_end): with a work list, the run of entries that
+// continue the same column plane by plane.
+__device__ __forceinline__ StreamSeg stream_segment(const SlabParams &p, int pos, int pos_end) {
   StreamSeg s;
+  const int step = p.items ? __ldg(p.items + pos) : pos;
   const int col = step / p.D;
   s.t0 = step - col * p.D;
-  const int left = step_end - step;
-  s.t1 = s.t0 + left < p.D ? s.t0 + left : p.D;
+  if (p.items) {
+    int len = 1;
+    while (pos + len < pos_end && s.t0 + len < p.D && __ldg(p.items + pos + len) == step + len) ++len;
+    s.t1 = s.t0 + len;
+  } else {
+    const int left = pos_end - pos;
+    s.t1 = s.t0 + left < p.D ? s.t0 + left : p.D;
+  }
   const int per_sample = p.cols_w * p.cols_h;
   s.sample = col / per_sample;
   const int r = col - s.sample * per_sample;
@@ -642,8 +661,11 @@ conv3d_stream32_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
   tmem_base = __shfl_sync(0xffffffffu, tmem_base, 0);
 
-  const int step_begin = (int)(((long long)blockIdx.x * p.steps_total) / gridDim.x);
-  const int step_end = (int)(((long long)(blockIdx.x + 1) * p.steps_total) / gridDim.x);
+  // positions in the work list, if there is one (a step's output plane depends only on planes t-1, t, t+1 and the
+  // order of their MMAs, not on where its segment starts)
+  const int steps_total = p.items ? *p.count : p.steps_total;
+  const int step_begin = (int)(((long long)blockIdx.x * steps_total) / gridDim.x);
+  const int step_end = (int)(((long long)(blockIdx.x + 1) * steps_total) / gridDim.x);
 
   if (warp == SL_B_WARP) {
     if (lane == 0) {  // the whole filter, once: 27 boxes of 32 rows x 64 channels
@@ -843,6 +865,7 @@ int slab_plan_fill(dram_conv_plan *pl, const dram_conv_desc *d, const void *src1
       return DRAM_E_ARG;
     }
   }
+  sp.items = sp.count = nullptr;
   sp.epi = epi;
   // Cin 64 -> Cout 32 with one source (us3): weights-resident streaming kernel; DRAM_B200_US3=ring keeps the items
   const char *us3 = getenv("DRAM_B200_US3");
@@ -897,8 +920,21 @@ int slab_plan_fill(dram_conv_plan *pl, const dram_conv_desc *d, const void *src1
   return rc;
 }
 
-int slab_plan_run(const dram_conv_plan *pl, int ctas, cudaStream_t st) {
+int slab_plan_listable(const dram_conv_plan *pl) { return pl->sp.stream || (!pl->sp.up2x && pl->block_n == 64); }
+
+// The work items of a listable plan: plane-ring items of 8 x 16 x 4 voxels or plane steps of 8 x 16 x 1 voxels, both
+// numbered with D fastest.
+int slab_plan_worklist(const dram_conv_plan *pl, const uint32_t *bits, int radius, uint8_t *flags, int *list, int *count,
+                       cudaStream_t st) {
+  const SlabParams &sp = pl->sp;
+  return worklist_build(bits, sp.n, sp.D, sp.H, sp.W, SL_W, SL_H, sp.stream ? 1 : slab_group(pl->block_n), 1, radius,
+                        flags, list, count, sp.stream ? sp.steps_total : sp.items_total, st);
+}
+
+int slab_plan_run(const dram_conv_plan *pl, int ctas, cudaStream_t st, const int *items, const int *count) {
   SlabParams sp = pl->sp;
+  sp.items = items;
+  sp.count = count;
   sp.epi = with_sat_counter(sp.epi);
   if (sp.stream) {
     if (sp.steps_total < ctas) ctas = sp.steps_total;

@@ -428,7 +428,10 @@ int pair_plan_run(const dram_conv_plan *pl, int ctas, cudaStream_t st);
 int slab_plan_supported(const dram_conv_desc *d);
 int slab_plan_fill(dram_conv_plan *pl, const dram_conv_desc *d, const void *src1, const void *src2,
                    const void *weight, const EpiParams &epi);
-int slab_plan_run(const dram_conv_plan *pl, int ctas, cudaStream_t st);
+int slab_plan_run(const dram_conv_plan *pl, int ctas, cudaStream_t st, const int *items, const int *count);
+int slab_plan_listable(const dram_conv_plan *pl);
+int slab_plan_worklist(const dram_conv_plan *pl, const uint32_t *bits, int radius, uint8_t *flags, int *list, int *count,
+                       cudaStream_t st);
 
 }  // namespace dram
 
@@ -771,7 +774,7 @@ extern "C" int dram_conv3d_run(const dram_conv_plan *plan, int32_t max_ctas, voi
   int ctas = sm_count();
   if (max_ctas > 0 && max_ctas < ctas) ctas = max_ctas;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (plan->kind == 1) return slab_plan_run(plan, ctas, st);
+  if (plan->kind == 1) return slab_plan_run(plan, ctas, st, nullptr, nullptr);
   if (plan->pair) return pair_plan_run(plan, ctas, st);
   if (plan->p.total_tiles < ctas) ctas = plan->p.total_tiles;
   dim3 grid(ctas);
@@ -791,4 +794,28 @@ extern "C" int dram_conv3d_run(const dram_conv_plan *plan, int32_t max_ctas, voi
   }
   DRAM_CHECK_LAUNCH("conv3d_umma_kernel launch");
   return DRAM_OK;
+}
+
+static bool conv_listable(const dram_conv_plan *plan) { return plan->kind == 1 && slab_plan_listable(plan); }
+
+extern "C" int dram_conv3d_worklist_size(const dram_conv_plan *plan, int32_t *entries) {
+  DRAM_REQUIRE(plan && entries, "dram_conv3d_worklist_size: null argument");
+  *entries = conv_listable(plan) ? (plan->sp.stream ? plan->sp.steps_total : plan->sp.items_total) : 0;
+  return DRAM_OK;
+}
+
+extern "C" int dram_conv3d_worklist(const dram_conv_plan *plan, const uint32_t *support, int32_t radius, uint8_t *flags,
+                                    int32_t *items, int32_t *count, void *stream) {
+  DRAM_REQUIRE(plan, "dram_conv3d_worklist: null plan");
+  DRAM_REQUIRE(conv_listable(plan), "dram_conv3d_worklist: this plan's kernel takes no work list");
+  return slab_plan_worklist(plan, support, radius, flags, items, count, reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int dram_conv3d_run_listed(const dram_conv_plan *plan, const int32_t *items, const int32_t *count,
+                                      int32_t max_ctas, void *stream) {
+  DRAM_REQUIRE(plan && items && count, "dram_conv3d_run_listed: null argument");
+  DRAM_REQUIRE(conv_listable(plan), "dram_conv3d_run_listed: this plan's kernel takes no work list");
+  int ctas = sm_count();
+  if (max_ctas > 0 && max_ctas < ctas) ctas = max_ctas;
+  return slab_plan_run(plan, ctas, reinterpret_cast<cudaStream_t>(stream), items, count);
 }

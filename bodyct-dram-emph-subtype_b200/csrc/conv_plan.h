@@ -57,6 +57,9 @@ struct SlabParams {
   // weights-resident streaming kernel (Cin 64 -> Cout 32): work = (column, output plane) steps
   int stream;                  // 0 / 1
   int steps_total;             // n * cols_w * cols_h * D
+  // optional work list (dram_conv3d_run_listed): the kernel runs items / steps items[0 .. *count) instead of all of
+  // them; null = every item
+  const int *items, *count;
   EpiParams epi;
 };
 

@@ -40,6 +40,7 @@ struct UpParams {
   int tiles_w, tiles_h, tiles_d, tiles_per_sample, total_tiles;
   float sd, sh, sw;                  // ATen source scales
   int is_f16;                        // storage type of in / out (the interpolation matrix is always fp16)
+  const int *items, *count;          // optional work list: tiles items[0 .. *count) instead of all (null = all)
 };
 
 struct UpTile {
@@ -114,13 +115,16 @@ upsample2x_umma_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
   tmem_base = __shfl_sync(0xffffffffu, tmem_base, 0);
+  // CTA b runs positions b, b + grid, ... of the work list (of all tiles without one)
+  const int total = p.items ? *p.count : p.total_tiles;
+  auto tile_at = [&](int i) { return p.items ? __ldg(p.items + i) : i; };
 
   if (warp == U_PRODUCER_WARP) {
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-        const UpTile t = decode_up_tile(p, tile);
+      for (int i = blockIdx.x; i < total; i += gridDim.x) {
+        const UpTile t = decode_up_tile(p, tile_at(i));
         for (int c = 0; c < p.chunks; ++c) {
           mbar_wait(b_empty(stage), phase ^ 1u);
           mbar_expect_tx(b_full(stage), U_B_BYTES);
@@ -137,7 +141,7 @@ upsample2x_umma_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_
     const uint32_t idesc = make_idesc_up(64, p.is_f16);
     int stage = 0, acc = 0, wi = 0;
     uint32_t phase = 0, acc_phase = 0, w_phase = 0;
-    for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
+    for (int i = blockIdx.x; i < total; i += gridDim.x) {
       mbar_wait(w_full(wi), w_phase);
       tcgen05_fence_after();
       for (int c = 0; c < p.chunks; ++c) {
@@ -228,8 +232,8 @@ upsample2x_umma_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_
     };
     int wi = 0;
     uint32_t w_phase = 0;
-    for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-      const UpTile t = decode_up_tile(p, tile);
+    for (int i = blockIdx.x; i < total; i += gridDim.x) {
+      const UpTile t = decode_up_tile(p, tile_at(i));
       mbar_wait(w_empty(wi), w_phase ^ 1u);
       if (wi == 0) generate(t, w_addr(0), prev0);
       else generate(t, w_addr(1), prev1);
@@ -245,8 +249,8 @@ upsample2x_umma_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_
     const int row = warp * 32 + lane;
     int acc = 0, gi = 0;
     uint32_t acc_phase = 0;
-    for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-      const UpTile t = decode_up_tile(p, tile);
+    for (int i = blockIdx.x; i < total; i += gridDim.x) {
+      const UpTile t = decode_up_tile(p, tile_at(i));
       for (int c = 0; c < p.chunks; ++c, ++gi) {
         const int b = gi & 1;
         mbar_wait(t_full(acc), acc_phase);
@@ -367,13 +371,42 @@ extern "C" int dram_upsample2x_plan_destroy(dram_upsample_plan *plan) {
   return DRAM_OK;
 }
 
-extern "C" int dram_upsample2x_plan_run(const dram_upsample_plan *plan, int32_t max_ctas, void *stream) {
-  DRAM_REQUIRE(plan, "dram_upsample2x_plan_run: null plan");
+static int upsample_launch(const dram_upsample_plan *plan, const int *items, const int *count, int32_t max_ctas,
+                           void *stream) {
   int ctas = sm_count();
   if (max_ctas > 0 && max_ctas < ctas) ctas = max_ctas;
   if (plan->p.total_tiles < ctas) ctas = plan->p.total_tiles;
+  UpParams p = plan->p;
+  p.items = items;
+  p.count = count;
   upsample2x_umma_kernel<<<ctas, U_THREADS, U_SMEM_BYTES, reinterpret_cast<cudaStream_t>(stream)>>>(
-      plan->map_in, plan->map_out, plan->p);
+      plan->map_in, plan->map_out, p);
   DRAM_CHECK_LAUNCH("upsample2x_umma_kernel launch");
   return DRAM_OK;
+}
+
+extern "C" int dram_upsample2x_plan_run(const dram_upsample_plan *plan, int32_t max_ctas, void *stream) {
+  DRAM_REQUIRE(plan, "dram_upsample2x_plan_run: null plan");
+  return upsample_launch(plan, nullptr, nullptr, max_ctas, stream);
+}
+
+extern "C" int dram_upsample2x_worklist_size(const dram_upsample_plan *plan, int32_t *entries) {
+  DRAM_REQUIRE(plan && entries, "dram_upsample2x_worklist_size: null argument");
+  *entries = plan->p.total_tiles;
+  return DRAM_OK;
+}
+
+// Work items: the 8 x 4 x 4 output bricks, numbered with W fastest.
+extern "C" int dram_upsample2x_worklist(const dram_upsample_plan *plan, const uint32_t *support, int32_t radius,
+                                        uint8_t *flags, int32_t *tiles, int32_t *count, void *stream) {
+  DRAM_REQUIRE(plan, "dram_upsample2x_worklist: null plan");
+  const UpParams &p = plan->p;
+  return worklist_build(support, p.n, p.D, p.H, p.W, U_TW, U_TH, U_TD, 0, radius, flags, tiles, count, p.total_tiles,
+                        reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int dram_upsample2x_plan_run_listed(const dram_upsample_plan *plan, const int32_t *tiles,
+                                               const int32_t *count, int32_t max_ctas, void *stream) {
+  DRAM_REQUIRE(plan && tiles && count, "dram_upsample2x_plan_run_listed: null argument");
+  return upsample_launch(plan, tiles, count, max_ctas, stream);
 }

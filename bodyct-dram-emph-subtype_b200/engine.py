@@ -51,6 +51,8 @@ class Med3DEngine:
         self.steps = []
         self.conv_flops = 0
         self._graph = None
+        self._graph_restricted = None
+        self._restricted = None   # (support scratch, support bits, launch list) of run_network(active_ess=...)
         self._sat_counter = torch.zeros(1, dtype=torch.int32, device=device)
         self._sat_checked_epoch = None
         self.last_saturation_count = None   # result of the latest probed pass (None: never probed)
@@ -191,8 +193,9 @@ class Med3DEngine:
             if k4_umma and src.shape[4] % 64 == 0:
                 plan = ops.Upsample2xPlan(src, out=dst)
                 self.steps.append(_Step(name, plan.run))
-            else:
-                self.steps.append(_Step(name, lambda: ops.upsample2x(src, out=dst)))
+                return plan
+            self.steps.append(_Step(name, lambda: ops.upsample2x(src, out=dst)))
+            return None
 
         cb = m.us1.conv_blocks
         # us1.0 (Cin = 512e + 64 -> 64): by default commuted (K13) — 27 channel-mixing products of x4 at LOW
@@ -209,13 +212,17 @@ class Med3DEngine:
             t = self._add_conv("us1.0", self.up1, self._conv_bn("us1.0", cb[0][0], cb[0][1]), x2=x1).out
         xup1 = self._add_conv("us1.1", t, self._conv_bn("us1.1", cb[1][0], cb[1][1])).out
         cb = m.us2.conv_blocks
+        # the full-resolution stage and how far (in voxels) beyond the dRAM's support each step's output is read
+        decoder = []
         if fused_up:
-            t = self._add_conv("us2.0", xup1, self._conv_bn("us2.0", cb[0][0], cb[0][1]), x2=x, upsample_x1=True).out
+            us20 = self._add_conv("us2.0", xup1, self._conv_bn("us2.0", cb[0][0], cb[0][1]), x2=x, upsample_x1=True)
         else:
             self.up2 = torch.empty((B, D1, H1, W1, 64), dtype=bf, device=dev)
-            add_upsample("us2.upsample", xup1, self.up2)
-            t = self._add_conv("us2.0", self.up2, self._conv_bn("us2.0", cb[0][0], cb[0][1]), x2=x).out
-        xup2 = self._add_conv("us2.1", t, self._conv_bn("us2.1", cb[1][0], cb[1][1])).out
+            decoder.append(("us2.upsample", add_upsample("us2.upsample", xup1, self.up2), 3, self.up2))
+            us20 = self._add_conv("us2.0", self.up2, self._conv_bn("us2.0", cb[0][0], cb[0][1]), x2=x)
+        us21 = self._add_conv("us2.1", us20.out, self._conv_bn("us2.1", cb[1][0], cb[1][1]))
+        decoder += [("us2.0", us20, 2, us20.out), ("us2.1", us21, 1, us21.out)]
+        t, xup2 = us20.out, us21.out
         # ---- us3 + heads fused
         head_ch = tuple(fc.weight.shape[0] for fc in m.fcs)
 
@@ -238,6 +245,15 @@ class Med3DEngine:
                              store_out=False)
         self.conv_flops += 2 * B * D1 * H1 * W1 * 32 * sum(head_ch)
         self.dense = us3.head_outs
+        decoder.append(("us3+heads", us3, 0, None))
+        self._decoder = decoder
+        # A restricted run writes only around the dRAM's support; the other voxels of these buffers are read (as halo of
+        # active items, and by K7's weight-0 corners) but never reach a result: zeros until a run overwrites them.
+        for _, _, _, buf in decoder:
+            if buf is not None:
+                buf.zero_()
+        for buf in self.dense:
+            buf.zero_()
         self.half_dims = (D1, H1, W1)
         self._plans_alive = [s.fn for s in self.steps]
 
@@ -308,9 +324,43 @@ class Med3DEngine:
         w, b, m = self.stem_weights
         return lambda: ops.stem_conv7(img, w, b, m, out=self.stem_out)
 
-    def run_network(self, first=None):
+    def _restricted_tail(self):
+        """Launches of the recorded sequence after the first step, with the full-resolution decoder steps restricted to
+        the work items the dRAM of the ess mask reaches (needs `self._restricted` filled by `_support`)."""
+        for fn in self._restricted[2]:
+            fn()
+
+    def _support(self, ess):
+        """Eager part of a restricted run: the support bits of `ess` uint8 [B, D, H, W] on the decoder grid."""
+        if tuple(ess.shape) != (self.batch,) + self.dims or ess.dtype != torch.uint8 or not ess.is_contiguous():
+            raise ValueError(f"active_ess: expected contiguous uint8 {(self.batch,) + self.dims}, got "
+                             f"{ess.dtype} {tuple(ess.shape)}")
+        if self._restricted is None:
+            B, (D, H, W), (d, h, w) = self.batch, self.dims, self.half_dims
+            words = (w + 31) // 32
+            rows = torch.empty((B, D, H, words), dtype=torch.int32, device=self.device)
+            support = torch.empty((B, d, h, words), dtype=torch.int32, device=self.device)
+            lists, listed = [], {}
+            for name, plan, radius, _ in self._decoder:
+                size = plan.worklist_size() if plan is not None else 0
+                if size == 0:
+                    continue   # a kernel without work lists (selected by a DRAM_B200_* experiment switch) stays dense
+                flags = torch.empty(size, dtype=torch.uint8, device=self.device)
+                items = torch.empty(size, dtype=torch.int32, device=self.device)
+                count = torch.empty(1, dtype=torch.int32, device=self.device)
+                lists.append(lambda plan=plan, r=radius, f=flags, i=items, c=count: plan.build_worklist(support, r, f, i, c))
+                listed[name] = lambda plan=plan, i=items, c=count: plan.run_listed(i, c)
+            self._restricted = (rows, support, lists + [listed.get(st.name, st.fn) for st in self.steps[1:]])
+        rows, support, _ = self._restricted
+        ops.decoder_support(ess, self.half_dims, rows=rows, out=support)
+
+    def run_network(self, first=None, active_ess=None):
         """The recorded launch sequence on `self.image` -> `self.dense` (engine-owned), on the current stream.
         `first` replaces the first step (see `hu_stem`); it is launched eagerly, the rest replays as a graph.
+        `active_ess` (uint8 [B, D, H, W], the ess mask K7 will apply): the dense maps are computed only where K7 reads
+        them for this mask — the full-resolution decoder steps run the work items that reach those voxels, with the same
+        arithmetic, so the dRAM is bit-identical to a dense run's; elsewhere the maps hold stale finite values.  The
+        mask is read by an eager launch in front of the graph (its address changes from call to call).
 
         * fp16 storage: the first pass after the weights changed (`DRAM_B200_SAT_CHECK=first`, default; `always` /
           `off`) runs with the library's saturation probe on and raises `ops.ActivationOverflow` if any convolution
@@ -326,7 +376,7 @@ class Med3DEngine:
             self._sat_counter.zero_()
             ops.check(lib.dram_set_saturation_counter(ops._p(self._sat_counter)), "dram_set_saturation_counter")
             try:
-                self._launch_steps(first)
+                self._launch_steps(first)   # dense, also for a restricted call: the probe covers every voxel
             finally:
                 lib.dram_set_saturation_counter(None)
             clamped = int(self._sat_counter.item())
@@ -337,18 +387,24 @@ class Med3DEngine:
                     "checkpoint/input needs bf16 storage (model.act_dtype = torch.bfloat16 or DRAM_B200_DTYPE=bf16)")
             self._sat_checked_epoch = self._weights_epoch
             return self.dense
+        tail = self._launch_tail
+        if active_ess is not None:
+            self._support(active_ess)
+            tail = self._restricted_tail
         if not ops.graphs_enabled() or torch.cuda.is_current_stream_capturing():
-            self._launch_steps(first)
+            (first or self.steps[0].fn)()
+            tail()
             return self.dense
         (first or self.steps[0].fn)()   # the stem reads a caller-owned buffer in the HU variant: outside the graph
-        if self._graph is None:
-            self._launch_tail()  # warm-up outside the capture (lazy function attributes, module loading)
+        attr = "_graph" if active_ess is None else "_graph_restricted"
+        if getattr(self, attr) is None:
+            tail()  # warm-up outside the capture (lazy function attributes, module loading)
             torch.cuda.current_stream(self.device).synchronize()
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph, capture_error_mode="thread_local"):
-                self._launch_tail()
-            self._graph = graph
-        self._graph.replay()
+                tail()
+            setattr(self, attr, graph)
+        getattr(self, attr).replay()
         return self.dense
 
     def load_image(self, image):

@@ -275,12 +275,13 @@ class ScanRegLightningModule(_ScanModule):
                                    "classification one; use ScanCLSLightningModule for med3d/med3d18/med3d50")
             B, D, H, W = image.shape
             eng = self.model.eval().engine(B, (D, H, W), image.device)
-            # the lobe-masked means of forward() are not used here (quirk Q2): no K6
+            # the lobe-masked means of forward() are not used here (quirk Q2): no K6.  K7 reads the dense maps only
+            # around `ess`: the full-resolution decoder runs there only (active_ess)
             if hasattr(eng, "stem_weights"):
-                dense = eng.run_network(first=eng.image_stem(image))  # the stem reads the batch's image in place
+                dense = eng.run_network(first=eng.image_stem(image), active_ess=ess)  # the stem reads the image in place
             else:
                 eng.load_image(image)
-                dense = eng.run_network()
+                dense = eng.run_network(active_ess=ess)
             cle, pse, pct = ops.dram_upsample_mask(dense[0], dense[1], ess, lungs, (D, H, W),
                                                    per_sample_denominator=self.per_sample_percentage)
             out = {
@@ -316,13 +317,13 @@ class ScanRegLightningModule(_ScanModule):
                 import os
 
                 fuse_window = os.environ.get("DRAM_B200_FUSE_WINDOW", "0").lower() in ("1", "on", "true", "yes")
+            lungs, ess = _as_u8(lung_mask), _as_u8(ess_mask)
             if fuse_window and hasattr(eng, "stem_weights"):
                 lut, _ = ops.window_lut(hu)  # statistics are per volume (intensity_transforms.py:104-114)
-                dense = eng.run_network(first=eng.hu_stem(hu, lut))
+                dense = eng.run_network(first=eng.hu_stem(hu, lut), active_ess=ess)
             else:
                 ops.window_standardize(hu, out=eng.image, batched=True)
-                dense = eng.run_network()
-            lungs, ess = _as_u8(lung_mask), _as_u8(ess_mask)
+                dense = eng.run_network(active_ess=ess)
             cle, pse, pct = ops.dram_upsample_mask(dense[0], dense[1], ess, lungs, (D, H, W),
                                                    per_sample_denominator=self.per_sample_percentage)
             out = {"cle_dense_outs": cle, "pse_dense_outs": pse, "cle_precentages": pct[0],

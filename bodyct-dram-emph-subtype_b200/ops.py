@@ -210,6 +210,24 @@ class Conv3dPlan:
         check(self._lib.dram_conv3d_run(self._handle, max_ctas, _stream()), "dram_conv3d_run")
         return self.out
 
+    def worklist_size(self):
+        """Number of work items if the plan's kernel takes a work list (`run_listed`), else 0."""
+        n = C.c_int32()
+        check(self._lib.dram_conv3d_worklist_size(self._handle, C.byref(n)), "dram_conv3d_worklist_size")
+        return n.value
+
+    def build_worklist(self, support, radius, flags, items, count):
+        """Items whose output box grown by `radius` meets `support` (`decoder_support` on the output grid) ->
+        items int32 [worklist_size()] (ascending) and count int32 [1], on the device; flags: uint8 scratch."""
+        check(self._lib.dram_conv3d_worklist(self._handle, _p(support), radius, _p(flags), _p(items), _p(count),
+                                             _stream()), "dram_conv3d_worklist")
+
+    def run_listed(self, items, count, max_ctas=0):
+        """`run` restricted to the listed work items; the other output voxels keep their values."""
+        check(self._lib.dram_conv3d_run_listed(self._handle, _p(items), _p(count), max_ctas, _stream()),
+              "dram_conv3d_run_listed")
+        return self.out
+
     def __del__(self):
         h = getattr(self, "_handle", None)
         if h:
@@ -404,6 +422,21 @@ class Upsample2xPlan:
         check(self._lib.dram_upsample2x_plan_run(self._handle, max_ctas, _stream()), "dram_upsample2x_plan_run")
         return self.out
 
+    def worklist_size(self):
+        n = C.c_int32()
+        check(self._lib.dram_upsample2x_worklist_size(self._handle, C.byref(n)), "dram_upsample2x_worklist_size")
+        return n.value
+
+    def build_worklist(self, support, radius, flags, items, count):
+        """As Conv3dPlan.build_worklist, over the 8x4x4 output bricks."""
+        check(self._lib.dram_upsample2x_worklist(self._handle, _p(support), radius, _p(flags), _p(items), _p(count),
+                                                 _stream()), "dram_upsample2x_worklist")
+
+    def run_listed(self, items, count, max_ctas=0):
+        check(self._lib.dram_upsample2x_plan_run_listed(self._handle, _p(items), _p(count), max_ctas, _stream()),
+              "dram_upsample2x_plan_run_listed")
+        return self.out
+
     def __del__(self):
         h = getattr(self, "_handle", None)
         if h:
@@ -412,6 +445,26 @@ class Upsample2xPlan:
             except Exception:
                 pass
             self._handle = None
+
+
+def decoder_support(ess, half_dims, rows=None, out=None):
+    """The decoder-grid voxels K7 reads for `ess` uint8 [N, D, H, W]: bit mask int32 [N, d, h, ceil(w/32)] over the
+    grid `half_dims` = (d, h, w) (see dram_decoder_support).  `rows` / `out`: optional preallocated scratch / result."""
+    lib = _capi.load()
+    _need(ess, torch.uint8, "decoder_support ess", 4)
+    n, D, H, W = ess.shape
+    d, h, w = half_dims
+    words = (w + 31) // 32
+    if rows is None:
+        rows = torch.empty((n, D, H, words), dtype=torch.int32, device=ess.device)
+    if out is None:
+        out = torch.empty((n, d, h, words), dtype=torch.int32, device=ess.device)
+    _need(rows, torch.int32, "decoder_support rows", 4)
+    _need(out, torch.int32, "decoder_support out", 4)
+    if tuple(rows.shape) != (n, D, H, words) or tuple(out.shape) != (n, d, h, words):
+        raise ValueError("decoder_support: scratch / output shape mismatch")
+    check(lib.dram_decoder_support(_p(ess), n, D, H, W, d, h, w, _p(rows), _p(out), _stream()), "dram_decoder_support")
+    return out
 
 
 def upconv_axis(x, axis, groups, out=None):

@@ -155,6 +155,20 @@ int dram_conv3d_plan_info(const dram_conv_plan *plan, int64_t *flops, int32_t *m
  * 64-channel chunk) stage it executes.  Differs from the algorithmic 2*M*N*K of dram_conv3d_plan_info by the taps
  * skipped inside the zero padding (dilated layers: fewer) and by the padding of border tiles (more). */
 int dram_conv3d_plan_executed_flops(const dram_conv_plan *plan, int64_t *flops);
+/*
+ * Work lists (decoder_mask.cu): a run restricted to the work items whose output box, grown by `radius` voxels, meets
+ * the support bit mask of dram_decoder_support, whose grid must be the plan's output grid.  Only the 64-channel
+ * plane-ring kernel with its sources at full resolution and the 64 -> 32 streaming kernel take a list:
+ * dram_conv3d_worklist_size gives 0 for every other plan, otherwise the number of work items (the capacity of
+ * `items`; `flags` is scratch of as many bytes).  dram_conv3d_worklist writes the ascending item indices and their
+ * number to device memory; dram_conv3d_run_listed reads both on the device (the grid is that of dram_conv3d_run, so
+ * the launch is graph-capturable) and computes every listed item exactly as dram_conv3d_run does.
+ */
+int dram_conv3d_worklist_size(const dram_conv_plan *plan, int32_t *entries);
+int dram_conv3d_worklist(const dram_conv_plan *plan, const uint32_t *support, int32_t radius, uint8_t *flags,
+                         int32_t *items, int32_t *count, void *stream);
+int dram_conv3d_run_listed(const dram_conv_plan *plan, const int32_t *items, const int32_t *count, int32_t max_ctas,
+                           void *stream);
 
 
 /* ---- K2a: stem unfold (feeds K1 with taps 7x1x1, stride 2x1x1) --------- */
@@ -220,6 +234,21 @@ int dram_upsample2x_plan_create(const void *x, void *out, int32_t n, int32_t d, 
                                 int32_t c, int32_t dtype, dram_upsample_plan **plan);
 int dram_upsample2x_plan_destroy(dram_upsample_plan *plan);
 int dram_upsample2x_plan_run(const dram_upsample_plan *plan, int32_t max_ctas, void *stream);
+/* Work lists of the 8x4x4 output bricks, as dram_conv3d_worklist* (the support grid is the output grid). */
+int dram_upsample2x_worklist_size(const dram_upsample_plan *plan, int32_t *entries);
+int dram_upsample2x_worklist(const dram_upsample_plan *plan, const uint32_t *support, int32_t radius, uint8_t *flags,
+                             int32_t *tiles, int32_t *count, void *stream);
+int dram_upsample2x_plan_run_listed(const dram_upsample_plan *plan, const int32_t *tiles, const int32_t *count,
+                                    int32_t max_ctas, void *stream);
+
+/* ---- support of the dRAM on the decoder grid (decoder_mask.cu) ---------- */
+/*
+ * K7 reads the dense maps [n][d][h][w] only at the trilinear (align_corners=True) corners {i0, i1} per axis of the
+ * ess voxels (i1 included where its weight is 0).  Writes that set as bits: support[((s*d + z)*h + y)*words + x/32]
+ * bit x%32, words = ceil(w/32).  ess: uint8 [n][D][H][W]; rows: scratch of n*D*H*words uint32.
+ */
+int dram_decoder_support(const uint8_t *ess, int32_t n, int32_t D, int32_t H, int32_t W, int32_t d, int32_t h,
+                         int32_t w, uint32_t *rows, uint32_t *support, void *stream);
 
 /* ---- K13: the commuted convolution of an up-sampled tensor (med3d.py:83-89, first conv of us1) ---- */
 /*
