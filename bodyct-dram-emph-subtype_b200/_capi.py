@@ -61,6 +61,9 @@ SIGNATURES = {
     "dram_conv3d_run": (C.c_int, [_vp, _i32, _vp]),
     "dram_conv3d_plan_info": (C.c_int, [_vp, C.POINTER(_i64), _pi32, _pi32, _pi32, _pi32]),
     "dram_conv3d_plan_executed_flops": (C.c_int, [_vp, C.POINTER(_i64)]),
+    "dram_conv3d_plan_brick": (C.c_int, [_vp, _pi32, _pi32, _pi32, _pi32, _pi32]),
+    "dram_conv3d_plan_order_size": (C.c_int, [_vp, _pi32]),
+    "dram_conv3d_plan_set_order": (C.c_int, [_vp, _vp, _vp]),
     "dram_conv3d_worklist_size": (C.c_int, [_vp, _pi32]),
     "dram_conv3d_worklist": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp]),
     "dram_conv3d_run_listed": (C.c_int, [_vp, _vp, _vp, _i32, _vp]),

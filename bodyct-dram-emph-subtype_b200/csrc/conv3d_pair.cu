@@ -4,13 +4,14 @@
 // Why: with a 128-voxel tile every (tap, chunk) stage moves a 16 KiB activation brick and a 32 KiB weight tile
 // for 128 x 256 x 64 MACs — 48 KiB per 512 tensor-core clocks, ~56 % of the L2->SM peak on its own (ncu
 // l1tex__m_xbar2l1tex_read_bytes, profiles/conv_ncu_r1f.md) with only four stages (2048 clocks) of look-ahead.
-// Here one CTA computes TWO bricks (256 voxels) against the same weight tile:
-//   stage = [A brick 0 | A brick 1 | B] = 64 KiB for 2 x 128 x 256 x 64 MACs (1024 clocks): a third less
+// Here one CTA computes a brick of 256 voxels, two 128-row boxes, against the same weight tile:
+//   stage = [A box 0 | A box 1 | B] = 64 KiB for 2 x 128 x 256 x 64 MACs (1024 clocks): a third less
 //   operand traffic per MAC and three stages = 3072 clocks of look-ahead;
-//   accumulators: brick 0 in TMEM columns [0,256), brick 1 in [256,512) — all of TMEM, so the epilogue of a tile
+//   accumulators: box 0 in TMEM columns [0,256), box 1 in [256,512) — all of TMEM, so the epilogue of a tile
 //   is not overlapped with the next tile's MMAs; with K >= 108 chunks per tile that costs a few per cent;
-//   epilogue: eight warps, warps 0-3 drain brick 0 and warps 6-9 brick 1 (TMEM lane quarter = warp % 4).
-// A tap is skipped only when BOTH bricks lie entirely in the zero padding.
+//   epilogue: eight warps, warps 0-3 drain box 0 and warps 6-9 box 1 (TMEM lane quarter = warp % 4).
+// The brick (p.bw x p.bh x p.bd voxels of p.bn samples) is split into its two boxes along the sample axis when it
+// folds samples, else along one spatial axis.  A tap is skipped when the whole brick lies in the zero padding.
 //
 // Roles (320 threads): warps 0-3 / 6-9 epilogue, warp 4 lane 0 TMA producer, warp 5 MMA issuer (owns TMEM).
 #include "conv_plan.h"
@@ -28,29 +29,20 @@ static constexpr int P_PRODUCER_WARP = 4, P_MMA_WARP = 5;
 static constexpr int P_TMEM_COLS = 512;
 static constexpr int P_SMEM_BYTES = 1024 + P_STAGES * P_STAGE_BYTES + 256;
 
-// Brick b (0 / 1) of pair-tile `tile`: m-tile 2 * pair + b.  m_ok is false for the odd brick past the end
-// (its TMA loads are out of bounds in the sample dimension = zeros, its rows are never stored).
+// Origins of the two boxes of a brick: box 1 is box 0 moved by the half of the brick along its split axis.  A box
+// past the end of the volume or batch is loaded out of bounds (zeros) and its rows are never stored.
 struct PairCoord {
   TileCoord t[2];
-  bool m_ok[2];
 };
 __device__ __forceinline__ PairCoord decode_pair(const ConvKParams &p, int tile) {
   PairCoord pc;
-  const int n_tile = tile % p.num_n_tiles;
-  const int pair = tile / p.num_n_tiles;
-#pragma unroll
-  for (int b = 0; b < 2; ++b) {
-    const int m_tile = 2 * pair + b;
-    pc.m_ok[b] = m_tile < p.m_tiles_total;
-    pc.t[b] = decode_tile(p, m_tile * p.num_n_tiles + n_tile, P_BLOCK_N);
-  }
+  pc.t[0] = decode_tile(p, tile, P_BLOCK_N);
+  pc.t[1] = pc.t[0];
+  pc.t[1].w0 += p.bw - p.tw;  // the brick is twice the box along exactly one axis
+  pc.t[1].h0 += p.bh - p.th;
+  pc.t[1].d0 += p.bd - p.td;
+  pc.t[1].sample += p.bn - p.tn;
   return pc;
-}
-// A tap contributes nothing to a brick when the brick's whole input window lies in the zero padding.
-__device__ __forceinline__ bool brick_tap_is_padding(const ConvKParams &p, const TileCoord &t, int zd, int zh, int zw) {
-  return tap_is_padding(t.d0 * p.sd + zd * p.dd - p.pd, p.td, p.sd, p.Di) ||
-         tap_is_padding(t.h0 * p.sh + zh * p.dh - p.ph, p.th, p.sh, p.Hi) ||
-         tap_is_padding(t.w0 * p.sw + zw * p.dw - p.pw, p.tw, p.sw, p.Wi);
 }
 
 __global__ void __launch_bounds__(P_THREADS, 1)
@@ -96,12 +88,12 @@ conv3d_pair_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-        const PairCoord pc = decode_pair(p, tile);
+      for (int i = blockIdx.x; i < p.total_tiles; i += gridDim.x) {
+        const PairCoord pc = decode_pair(p, tile_at(p, i));
         for (int zd = 0; zd < p.kd; ++zd)
           for (int zh = 0; zh < p.kh; ++zh)
             for (int zw = 0; zw < p.kw; ++zw) {
-              if (brick_tap_is_padding(p, pc.t[0], zd, zh, zw) && brick_tap_is_padding(p, pc.t[1], zd, zh, zw)) continue;
+              if (brick_tap_is_padding(p, pc.t[0], zd, zh, zw)) continue;
               const int tap = (zd * p.kh + zh) * p.kw + zw;
               for (int ch = 0; ch < p.chunks_total; ++ch) {
                 mbar_wait(empty_bar(stage), phase ^ 1u);
@@ -132,15 +124,15 @@ conv3d_pair_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
     const uint32_t idesc = make_idesc_16bit(128, P_BLOCK_N, p.epi.is_f16);
     int stage = 0;
     uint32_t phase = 0, acc_phase = 0;
-    for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-      const PairCoord pc = decode_pair(p, tile);
+    for (int i = blockIdx.x; i < p.total_tiles; i += gridDim.x) {
+      const PairCoord pc = decode_pair(p, tile_at(p, i));
       mbar_wait(tmem_empty_bar, acc_phase ^ 1u);  // the epilogue has drained both accumulators
       tcgen05_fence_after();
       uint32_t accumulate = 0;
       for (int zd = 0; zd < p.kd; ++zd)
         for (int zh = 0; zh < p.kh; ++zh)
           for (int zw = 0; zw < p.kw; ++zw) {
-            if (brick_tap_is_padding(p, pc.t[0], zd, zh, zw) && brick_tap_is_padding(p, pc.t[1], zd, zh, zw)) continue;
+            if (brick_tap_is_padding(p, pc.t[0], zd, zh, zw)) continue;
             for (int ch = 0; ch < p.chunks_total; ++ch) {
               mbar_wait(full_bar(stage), phase);
               tcgen05_fence_after();
@@ -168,19 +160,20 @@ conv3d_pair_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
       acc_phase ^= 1u;
     }
   } else {
-    // ------------------------------- epilogue: warps 0-3 brick 0, warps 6-9 brick 1 -------------------------------
+    // ------------------------------- epilogue: warps 0-3 box 0, warps 6-9 box 1 -------------------------------
     const int quarter = warp & 3, brick = warp < 4 ? 0 : 1;
     const int row = quarter * 32 + lane;
     const int lw = row & (p.tw - 1);
     const int lh = (row >> p.tw_log2) & (p.th - 1);
-    const int ld = row >> (p.tw_log2 + p.th_log2);
+    const int ld = (row >> (p.tw_log2 + p.th_log2)) & (p.td - 1);
+    const int ls = row >> (p.tw_log2 + p.th_log2 + p.td_log2);
     uint32_t acc_phase = 0;
-    for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-      const PairCoord pc = decode_pair(p, tile);
+    for (int i = blockIdx.x; i < p.total_tiles; i += gridDim.x) {
+      const PairCoord pc = decode_pair(p, tile_at(p, i));
       const TileCoord &t = pc.t[brick];
-      const int od = t.d0 + ld, oh = t.h0 + lh, ow = t.w0 + lw;
-      const bool valid = pc.m_ok[brick] && (od < p.Do) && (oh < p.Ho) && (ow < p.Wo);
-      const uint16_t *res_row = residual_row(p.epi, valid, t.sample, od, oh, ow);
+      const int od = t.d0 + ld, oh = t.h0 + lh, ow = t.w0 + lw, os = t.sample + ls;
+      const bool valid = (os < p.n) && (od < p.Do) && (oh < p.Ho) && (ow < p.Wo);
+      const uint16_t *res_row = residual_row(p.epi, valid, os, od, oh, ow);
       mbar_wait(tmem_full_bar, acc_phase);
       tcgen05_fence_after();
       const uint32_t taddr = tmem_base + (uint32_t)(brick * P_BLOCK_N) + ((uint32_t)(quarter * 32) << 16);
@@ -191,7 +184,7 @@ conv3d_pair_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
         tmem_ld_32x32b_x32(taddr + (uint32_t)c0, v);
         const ResGroup next = load_residual_group(p.epi, c0 + 32 < P_BLOCK_N ? res_row : nullptr, t.n0 + c0 + 32);
         tmem_wait_ld();
-        if (valid) epilogue_group<false>(p.epi, v, t.n0 + c0, t.sample, od, oh, ow, res);
+        if (valid) epilogue_group<false>(p.epi, v, t.n0 + c0, os, od, oh, ow, res);
         res = next;
       }
       tcgen05_fence_before();
@@ -211,7 +204,7 @@ conv3d_pair_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_cons
 // ----------------------------------------------------------------------------------------
 // host (called from dram_conv3d_plan_create / dram_conv3d_run in conv3d_umma.cu)
 // ----------------------------------------------------------------------------------------
-int pair_plan_wanted(const dram_conv_desc *d, int block_n, int64_t k_chunks, int64_t m_tiles, int n_tiles) {
+int pair_plan_wanted(const dram_conv_desc *d, int block_n, int64_t k_chunks, int64_t pair_tiles) {
   // wide output, long K loop (the un-overlapped epilogue must stay a few per cent), no fused heads
   if (!(block_n == P_BLOCK_N && d->cout % P_BLOCK_N == 0 && k_chunks >= 64 && d->n_heads == 0 && d->store_out))
     return 0;
@@ -220,15 +213,10 @@ int pair_plan_wanted(const dram_conv_desc *d, int block_n, int64_t k_chunks, int
   // Measured on B200 (DESIGN.md): +3 % on layer4 (512->512, 216 chunks) once the 256-voxel tiles fill >= 6 waves;
   // with fewer, larger tiles the last wave's idle SMs cost more than the saved operand traffic gains (layer3 at
   // batch 4: -12 %, everything at batch 1: -10 %).
-  const int64_t pair_tiles = (m_tiles + 1) / 2 * n_tiles;
   return k_chunks >= 200 && pair_tiles >= 6LL * sm_count();
 }
 
 int pair_plan_fill(dram_conv_plan *pl) {
-  ConvKParams &p = pl->p;
-  p.m_tiles_total = pl->m_tiles;
-  const int64_t total = (int64_t)((pl->m_tiles + 1) / 2) * p.num_n_tiles;
-  p.total_tiles = (int)total;
   pl->pair = 1;
   pl->stages = P_STAGES;
   pl->smem_bytes = P_SMEM_BYTES;

@@ -1,8 +1,11 @@
 // K1 — conv3d as an implicit GEMM on the sm_100a tensor cores.
 //
 //   A (activations) : NDHWC bf16.  One TMA box load per (filter tap, 64-channel chunk)
-//                     fetches the tap-shifted [td][th][tw][64] brick of the input straight
+//                     fetches the tap-shifted [tn][td][th][tw][64] brick of the input straight
 //                     into the canonical K-major SWIZZLE_128B UMMA layout (128 rows x 128 B).
+//                     A brick may span tn samples at the same spatial position: they share their
+//                     padding taps, so small spatial extents can line up with a dilated filter's
+//                     padding while one box still fills all 128 rows.
 //                     Zero padding = TMA out-of-bounds fill; dilation = tap offset;
 //                     stride = tensor-map elementStrides.  A second tensor map supplies the
 //                     channels of the skip tensor, so cat([up(x), skip]) is never built
@@ -18,7 +21,8 @@
 //
 // Roles (192 threads): warps 0-3 epilogue (TMEM lane quarter = warp id), warp 4 lane 0 TMA
 // producer, warp 5 lane 0 MMA issuer (warp 5 also owns the TMEM allocation).
-// Persistent: grid <= #SMs, tile = blockIdx.x + i * gridDim.x, n-tile fastest.
+// Persistent: grid <= #SMs, tile = order[blockIdx.x + i * gridDim.x], n-tile fastest.  When bricks differ in cost,
+// the plan's order lists them by descending executed stages (stable), so no CTA is left with the last heavy tiles.
 // Filter taps whose whole brick lies in the zero padding are skipped by producer and issuer.
 #include "umma_common.cuh"
 #include "conv_plan.h"
@@ -116,17 +120,17 @@ conv3d_umma_kernel(const __grid_constant__ CUtensorMap map_a1,
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-        const TileCoord t = decode_tile(p, tile, BLOCK_N);
+      for (int i = blockIdx.x; i < p.total_tiles; i += gridDim.x) {
+        const TileCoord t = decode_tile(p, tile_at(p, i), BLOCK_N);
         for (int zd = 0; zd < p.kd; ++zd) {
           const int id0 = t.d0 * p.sd + zd * p.dd - p.pd;
-          if (tap_is_padding(id0, p.td, p.sd, p.Di)) continue;
+          if (tap_is_padding(id0, p.bd, p.sd, p.Di)) continue;
           for (int zh = 0; zh < p.kh; ++zh) {
             const int ih0 = t.h0 * p.sh + zh * p.dh - p.ph;
-            if (tap_is_padding(ih0, p.th, p.sh, p.Hi)) continue;
+            if (tap_is_padding(ih0, p.bh, p.sh, p.Hi)) continue;
             for (int zw = 0; zw < p.kw; ++zw) {
               const int iw0 = t.w0 * p.sw + zw * p.dw - p.pw;
-              if (tap_is_padding(iw0, p.tw, p.sw, p.Wi)) continue;
+              if (tap_is_padding(iw0, p.bw, p.sw, p.Wi)) continue;
               const int tap = (zd * p.kh + zh) * p.kw + zw;
               for (int ch = 0; ch < p.chunks_total; ++ch) {
                 mbar_wait(empty_bar(stage), phase ^ 1u);
@@ -157,18 +161,18 @@ conv3d_umma_kernel(const __grid_constant__ CUtensorMap map_a1,
       uint32_t phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-        const TileCoord t = decode_tile(p, tile, BLOCK_N);
+      for (int i = blockIdx.x; i < p.total_tiles; i += gridDim.x) {
+        const TileCoord t = decode_tile(p, tile_at(p, i), BLOCK_N);
         mbar_wait(tmem_empty_bar(acc), acc_phase ^ 1u);
         tcgen05_fence_after();
         const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BLOCK_N);
         uint32_t accumulate = 0;
         for (int zd = 0; zd < p.kd; ++zd) {
-          if (tap_is_padding(t.d0 * p.sd + zd * p.dd - p.pd, p.td, p.sd, p.Di)) continue;
+          if (tap_is_padding(t.d0 * p.sd + zd * p.dd - p.pd, p.bd, p.sd, p.Di)) continue;
           for (int zh = 0; zh < p.kh; ++zh) {
-            if (tap_is_padding(t.h0 * p.sh + zh * p.dh - p.ph, p.th, p.sh, p.Hi)) continue;
+            if (tap_is_padding(t.h0 * p.sh + zh * p.dh - p.ph, p.bh, p.sh, p.Hi)) continue;
             for (int zw = 0; zw < p.kw; ++zw) {
-              if (tap_is_padding(t.w0 * p.sw + zw * p.dw - p.pw, p.tw, p.sw, p.Wi)) continue;
+              if (tap_is_padding(t.w0 * p.sw + zw * p.dw - p.pw, p.bw, p.sw, p.Wi)) continue;
               for (int ch = 0; ch < p.chunks_total; ++ch) {
                 mbar_wait(full_bar(stage), phase);
                 tcgen05_fence_after();
@@ -218,7 +222,7 @@ conv3d_umma_kernel(const __grid_constant__ CUtensorMap map_a1,
     const int quarter = warp & 3, half = warp < 4 ? 0 : 1;
     const int row = quarter * 32 + lane;
     const bool storer = half == 0 && lane == 0;
-    // where the quarter's first row sits inside the tw x th x td brick
+    // where the quarter's first row sits inside the tw x th x td brick (staged plans: tn = 1, no tile order)
     const int row0 = quarter * 32;
     const int qw = row0 & (p.tw - 1), qh = (row0 >> p.tw_log2) & (p.th - 1), qd = row0 >> (p.tw_log2 + p.th_log2);
     const bool has_res = p.staged_res != 0;
@@ -278,14 +282,16 @@ conv3d_umma_kernel(const __grid_constant__ CUtensorMap map_a1,
     const int row = warp * 32 + lane;  // TMEM lane == row of the 128-voxel tile
     const int lw = row & (p.tw - 1);
     const int lh = (row >> p.tw_log2) & (p.th - 1);
-    const int ld = row >> (p.tw_log2 + p.th_log2);
+    const int ld = (row >> (p.tw_log2 + p.th_log2)) & (p.td - 1);
+    const int ls = row >> (p.tw_log2 + p.th_log2 + p.td_log2);
     int acc = 0;
     uint32_t acc_phase = 0;
-    for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-      const TileCoord t = decode_tile(p, tile, BLOCK_N);
-      const int od = t.d0 + ld, oh = t.h0 + lh, ow = t.w0 + lw;
-      const bool valid = (od < p.Do) && (oh < p.Ho) && (ow < p.Wo);
-      const uint16_t *res_row = residual_row(p.epi, valid, t.sample, od, oh, ow);
+    for (int i = blockIdx.x; i < p.total_tiles; i += gridDim.x) {
+      const TileCoord t = decode_tile(p, tile_at(p, i), BLOCK_N);
+      const int od = t.d0 + ld, oh = t.h0 + lh, ow = t.w0 + lw, os = t.sample + ls;
+      // rows of samples past the batch (a folded brick of a ragged batch) are zeros and never stored
+      const bool valid = (os < p.n) && (od < p.Do) && (oh < p.Ho) && (ow < p.Wo);
+      const uint16_t *res_row = residual_row(p.epi, valid, os, od, oh, ow);
       ResGroup res = load_residual_group(p.epi, res_row, t.n0);  // in flight while this warp waits for the accumulator
       mbar_wait(tmem_full_bar(acc), acc_phase);
       tcgen05_fence_after();
@@ -296,7 +302,7 @@ conv3d_umma_kernel(const __grid_constant__ CUtensorMap map_a1,
         tmem_ld_32x32b_x32(taddr + (uint32_t)c0, v);
         const ResGroup next = load_residual_group(p.epi, c0 + 32 < BLOCK_N ? res_row : nullptr, t.n0 + c0 + 32);
         tmem_wait_ld();
-        if (valid) epilogue_group<BLOCK_N == 32>(p.epi, v, t.n0 + c0, t.sample, od, oh, ow, res);
+        if (valid) epilogue_group<BLOCK_N == 32>(p.epi, v, t.n0 + c0, os, od, oh, ow, res);
         res = next;
       }
       tcgen05_fence_before();
@@ -338,9 +344,9 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// NDHWC activation tensor as a 5-D map (C, W, H, D, N); box = box_c channels x bw x bh x bd voxels.
+// NDHWC activation tensor as a 5-D map (C, W, H, D, N); box = box_c channels x bw x bh x bd voxels x bn samples.
 int encode_act_map(CUtensorMap *map, const void *base, int n, int d, int h, int w, int c, int box_c, int bw,
-                   int bh, int bd, int sw, int sh, int sd, int is_f16) {
+                   int bh, int bd, int sw, int sh, int sd, int is_f16, int bn) {
   EncodeTiledFn enc = get_encode_fn();
   if (!enc) {
     set_error("cuTensorMapEncodeTiled is not available (no CUDA driver?)");
@@ -351,15 +357,15 @@ int encode_act_map(CUtensorMap *map, const void *base, int n, int d, int h, int 
                         (cuuint64_t)d * h * w * c * 2};
   // With a traversal stride s the box spans (t-1)*s+1 input elements and lands t of them.
   cuuint32_t box[5] = {(cuuint32_t)box_c, (cuuint32_t)((bw - 1) * sw + 1),
-                       (cuuint32_t)((bh - 1) * sh + 1), (cuuint32_t)((bd - 1) * sd + 1), 1};
+                       (cuuint32_t)((bh - 1) * sh + 1), (cuuint32_t)((bd - 1) * sd + 1), (cuuint32_t)bn};
   cuuint32_t estr[5] = {1, (cuuint32_t)sw, (cuuint32_t)sh, (cuuint32_t)sd, 1};
   CUresult r = enc(map, is_f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5,
                    const_cast<void *>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(activation %dx%dx%dx%dx%d box %dx%dx%d stride %d,%d,%d) -> %d",
-              n, d, h, w, c, bw, bh, bd, sw, sh, sd, (int)r);
+    set_error("cuTensorMapEncodeTiled(activation %dx%dx%dx%dx%d box %dx%dx%dx%d stride %d,%d,%d) -> %d",
+              n, d, h, w, c, bw, bh, bd, bn, sw, sh, sd, (int)r);
     return DRAM_E_DRIVER;
   }
   return DRAM_OK;
@@ -419,8 +425,61 @@ static bool is_pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
 
 static int conv_out(int in, int k, int s, int d, int p) { return (in + 2 * p - d * (k - 1) - 1) / s + 1; }
 
+// True when a brick of `extent` outputs starting at input coordinate i0 reads only zero padding (as tap_is_padding).
+static bool host_tap_is_padding(int i0, int extent, int stride, int in_size) {
+  return (i0 + (extent - 1) * stride < 0) || (i0 >= in_size);
+}
+
+// Brick extents (bw x bh x bd voxels of bn samples), its tile count and the (tap, brick) stages it issues per n-tile
+// and 64-channel chunk; split = the axis (0 w, 1 h, 2 d, 3 sample) along which the pair kernel halves it.
+struct BrickChoice {
+  int bw, bh, bd, bn;
+  int64_t tiles, stages;
+  int split;
+};
+
+// Taps not skipped, summed over the bricks of one axis.  A tap is skipped when the brick reads only padding along
+// some axis, so a brick executes the product of its three per-axis counts and the sum over bricks factorises.
+static int64_t axis_taps(int out, int ext, int k, int s, int dil, int pad, int in) {
+  int64_t sum = 0;
+  for (int b0 = 0; b0 < out; b0 += ext)
+    for (int z = 0; z < k; ++z) sum += host_tap_is_padding(b0 * s + z * dil - pad, ext, s, in) ? 0 : 1;
+  return sum;
+}
+
+static BrickChoice brick_cost(const dram_conv_desc *d, int Do, int Ho, int Wo, int bw, int bh, int bd, int bn) {
+  const int64_t groups = ceil_div(d->n, bn);
+  BrickChoice c{bw, bh, bd, bn, 0, 0, bn > 1 ? 3 : 0};
+  c.tiles = groups * ceil_div(Wo, bw) * ceil_div(Ho, bh) * ceil_div(Do, bd);
+  c.stages = groups * axis_taps(Wo, bw, d->kw, d->sw, d->dw, d->pw, d->wi) *
+             axis_taps(Ho, bh, d->kh, d->sh, d->dh, d->ph, d->hi) * axis_taps(Do, bd, d->kd, d->sd, d->dd, d->pd, d->di);
+  return c;
+}
+
+// The brick of `voxels` voxels a plan runs: the unfolded `base` shape, or with `fold` the brick spanning
+// bn = 2, 4, ... samples (bn < 2n) with the fewest executed stages.  Ties go to fewer tiles, then to the unfolded
+// shape, then to fewer samples and wider rows.  Folded spatial extents are at least 2: a brick one voxel thick
+// would skip padding taps of dilation-1 filters too, for a few per cent of their stages, at the price of tiles
+// that differ from the layout those layers were tuned with.
+static BrickChoice choose_brick(const dram_conv_desc *d, int Do, int Ho, int Wo, int voxels, const BrickChoice &base,
+                                bool fold) {
+  BrickChoice best = base;
+  if (!fold) return best;
+  for (int bn = 2; bn < 2 * d->n && bn <= voxels / 8; bn *= 2) {
+    const int sp = voxels / bn;
+    for (int w = sp / 4; w >= 2; w /= 2)
+      for (int h = sp / w / 2; h >= 2; h /= 2) {
+        const int dd = sp / (w * h);
+        if (dd < 2 || (w - 1) * d->sw + 1 > 256 || (h - 1) * d->sh + 1 > 256 || (dd - 1) * d->sd + 1 > 256) continue;
+        const BrickChoice c = brick_cost(d, Do, Ho, Wo, w, h, dd, bn);
+        if (c.stages < best.stages || (c.stages == best.stages && c.tiles < best.tiles)) best = c;
+      }
+  }
+  return best;
+}
+
 // M256 tile kernel (conv3d_pair.cu)
-int pair_plan_wanted(const dram_conv_desc *d, int block_n, int64_t k_chunks, int64_t m_tiles, int n_tiles);
+int pair_plan_wanted(const dram_conv_desc *d, int block_n, int64_t k_chunks, int64_t pair_tiles);
 int pair_plan_fill(dram_conv_plan *pl);
 int pair_plan_run(const dram_conv_plan *pl, int ctas, cudaStream_t st);
 
@@ -445,6 +504,95 @@ extern "C" int dram_conv3d_out_dims(const dram_conv_desc *d, int32_t *dout, int3
   *hout = conv_out(d->hi, d->kh, d->sh, d->dh, d->ph);
   *wout = conv_out(d->wi, d->kw, d->sw, d->dw, d->pw);
   return DRAM_OK;
+}
+
+// brick_tap_is_padding (conv_plan.h) on the host, for brick m_tile of the plan
+static bool host_brick_tap_skipped(const ConvKParams &p, int m_tile, int zd, int zh, int zw) {
+  const int r = m_tile % p.tiles_per_sample;
+  const int iw = r % p.tiles_w, r2 = r / p.tiles_w, ih = r2 % p.tiles_h, id = r2 / p.tiles_h;
+  return host_tap_is_padding(id * p.bd * p.sd + zd * p.dd - p.pd, p.bd, p.sd, p.Di) ||
+         host_tap_is_padding(ih * p.bh * p.sh + zh * p.dh - p.ph, p.bh, p.sh, p.Hi) ||
+         host_tap_is_padding(iw * p.bw * p.sw + zw * p.dw - p.pw, p.bw, p.sw, p.Wi);
+}
+static int brick_taps(const ConvKParams &p, int m_tile) {
+  int taps = 0;
+  for (int zd = 0; zd < p.kd; ++zd)
+    for (int zh = 0; zh < p.kh; ++zh)
+      for (int zw = 0; zw < p.kw; ++zw) taps += host_brick_tap_skipped(p, m_tile, zd, zh, zw) ? 0 : 1;
+  return taps;
+}
+
+// Tile walk order of the persistent kernels.  When bricks execute different numbers of taps (padding skipped at the
+// borders), a grid-stride walk in index order leaves some CTAs with several heavy tiles more than others.  Walking the
+// tiles by descending cost instead hands the light border tiles out last.  The sort is stable, so the (majority of)
+// full-cost tiles keep the n-tile-fastest raster order whose neighbours share operands in L2.
+// A brick's cost is the product of its per-axis tap counts (all >= 1), so costs differ exactly when some axis has
+// bricks with different counts.
+static bool axis_uniform(int out, int ext, int k, int s, int dil, int pad, int in) {
+  int first = -1;
+  for (int b0 = 0; b0 < out; b0 += ext) {
+    int taps = 0;
+    for (int z = 0; z < k; ++z) taps += host_tap_is_padding(b0 * s + z * dil - pad, ext, s, in) ? 0 : 1;
+    if (first >= 0 && taps != first) return false;
+    first = taps;
+  }
+  return true;
+}
+static bool tile_costs_differ(const dram_conv_plan *pl) {
+  const ConvKParams &p = pl->p;
+  if (pl->kind != 0 || pl->staged || p.kd * p.kh * p.kw == 1) return false;
+  return !(axis_uniform(p.Wo, p.bw, p.kw, p.sw, p.dw, p.pw, p.Wi) && axis_uniform(p.Ho, p.bh, p.kh, p.sh, p.dh, p.ph, p.Hi) &&
+           axis_uniform(p.Do, p.bd, p.kd, p.sd, p.dd, p.pd, p.Di));
+}
+
+// The order itself is built on the device, into a buffer the caller owns (dram_conv3d_plan_set_order): a counting
+// sort by descending cost in one CTA.  Costs are at most 7^3 taps; a chunk of blockDim m-tiles at a time is placed
+// after every earlier m-tile of its cost, so the sort is stable.
+static constexpr int ORDER_THREADS = 256;
+static constexpr int ORDER_MAX_COST = 343;
+__device__ int device_brick_taps(const ConvKParams &p, int m_tile) {
+  const TileCoord t = decode_tile(p, m_tile * p.num_n_tiles, 0);
+  int taps = 0;
+  for (int zd = 0; zd < p.kd; ++zd)
+    for (int zh = 0; zh < p.kh; ++zh)
+      for (int zw = 0; zw < p.kw; ++zw) taps += brick_tap_is_padding(p, t, zd, zh, zw) ? 0 : 1;
+  return taps;
+}
+__global__ void __launch_bounds__(ORDER_THREADS) conv_tile_order_kernel(const ConvKParams p, int m_tiles, int *order) {
+  __shared__ int next[ORDER_MAX_COST + 1];  // first free position of each cost class
+  __shared__ int chunk_cost[ORDER_THREADS];
+  const int tid = threadIdx.x;
+  for (int c = tid; c <= ORDER_MAX_COST; c += ORDER_THREADS) next[c] = 0;
+  __syncthreads();
+  for (int m = tid; m < m_tiles; m += ORDER_THREADS) atomicAdd(&next[device_brick_taps(p, m)], 1);
+  __syncthreads();
+  if (tid == 0) {  // histogram -> exclusive prefix in descending cost
+    int pos = 0;
+    for (int c = ORDER_MAX_COST; c >= 0; --c) {
+      const int count = next[c];
+      next[c] = pos;
+      pos += count;
+    }
+  }
+  __syncthreads();
+  for (int m0 = 0; m0 < m_tiles; m0 += ORDER_THREADS) {
+    const int m = m0 + tid;
+    const int c = m < m_tiles ? device_brick_taps(p, m) : -1;
+    chunk_cost[tid] = c;
+    __syncthreads();
+    int rank = 0, later = 0;  // same-cost m-tiles of this chunk before / after this one
+    for (int j = 0; j < ORDER_THREADS; ++j) {
+      rank += (j < tid && chunk_cost[j] == c) ? 1 : 0;
+      later += (j > tid && chunk_cost[j] == c) ? 1 : 0;
+    }
+    if (c >= 0) {
+      const int pos = next[c] + rank;
+      for (int nt = 0; nt < p.num_n_tiles; ++nt) order[pos * p.num_n_tiles + nt] = m * p.num_n_tiles + nt;
+    }
+    __syncthreads();
+    if (c >= 0 && later == 0) next[c] += rank + 1;  // the last m-tile of its class in the chunk moves the class on
+    __syncthreads();
+  }
 }
 
 template <int BN, bool STAGED>
@@ -575,9 +723,10 @@ extern "C" int dram_conv3d_plan_create(const dram_conv_desc *d, const void *src1
   }
 
   // ---- per-tap TMA tile kernel ------------------------------------------------------------------
-  // Tile shape: caller's choice or the candidate with the fewest tiles.
+  // Spatial shape: caller's choice or the candidate with the fewest tiles.
   int tw = d->tw, th = d->th, td = d->td;
-  if (tw == 0 || th == 0 || td == 0) {
+  const bool auto_tile = tw == 0 || th == 0 || td == 0;
+  if (auto_tile) {
     static const int cand[][3] = {{8, 4, 4}, {4, 8, 4}, {4, 4, 8}, {8, 8, 2},  {8, 2, 8}, {2, 8, 8},
                                   {16, 4, 2}, {4, 16, 2}, {16, 2, 4}, {2, 16, 4}, {16, 8, 1}, {8, 16, 1},
                                   {32, 4, 1}, {4, 32, 1}, {32, 2, 2}, {16, 1, 8}, {128, 1, 1}};
@@ -603,38 +752,6 @@ extern "C" int dram_conv3d_plan_create(const dram_conv_desc *d, const void *src1
     return DRAM_E_ARG;
   }
 
-  pl->kind = 0;
-  ConvKParams &p = pl->p;
-  p.n = d->n; p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.Di = d->di; p.Hi = d->hi; p.Wi = d->wi;
-  p.tw = tw; p.th = th; p.td = td; p.tw_log2 = ilog2(tw); p.th_log2 = ilog2(th);
-  p.tiles_w = ceil_div(Wo, tw); p.tiles_h = ceil_div(Ho, th); p.tiles_d = ceil_div(Do, td);
-  p.tiles_per_sample = p.tiles_w * p.tiles_h * p.tiles_d;
-  p.num_n_tiles = d->cout / block_n;
-  int64_t total = (int64_t)p.tiles_per_sample * d->n * p.num_n_tiles;
-  if (total > 0x7fffffffLL) {
-    delete pl;
-    set_error("conv3d: too many tiles");
-    return DRAM_E_ARG;
-  }
-  p.total_tiles = (int)total;
-  p.kd = d->kd; p.kh = d->kh; p.kw = d->kw; p.sd = d->sd; p.sh = d->sh; p.sw = d->sw;
-  p.dd = d->dd; p.dh = d->dh; p.dw = d->dw; p.pd = d->pd; p.ph = d->ph; p.pw = d->pw;
-  p.chunks1 = d->c1 / BLOCK_K;
-  p.chunks_total = (d->c1 + d->c2) / BLOCK_K;
-  p.epi = epi;
-  pl->m_tiles = p.tiles_per_sample * d->n;
-  pl->n_tiles = p.num_n_tiles;
-
-  int rc = encode_act_map(&pl->map_a1, src1, d->n, d->di, d->hi, d->wi, d->c1, BLOCK_K, tw, th, td, d->sw,
-                          d->sh, d->sd, epi.is_f16);
-  if (rc == DRAM_OK) {
-    if (d->c2 > 0)
-      rc = encode_act_map(&pl->map_a2, src2, d->n, d->di, d->hi, d->wi, d->c2, BLOCK_K, tw, th, td, d->sw,
-                          d->sh, d->sd, epi.is_f16);
-    else
-      pl->map_a2 = pl->map_a1;
-  }
-  if (rc == DRAM_OK) rc = encode_weight_map(&pl->map_w, weight, d->cout, ktot, block_n, epi.is_f16);
   // Staged (shared memory + TMA) epilogue for the 1x1x1 convolutions: they are bound by the epilogue's global
   // accesses, which the direct path issues as one 16-byte access per lane and row.
   // The residual tile is a TMA box too: shortcut type A (fewer channels, strided read) falls out of the tensor
@@ -652,20 +769,70 @@ extern "C" int dram_conv3d_plan_create(const dram_conv_desc *d, const void *src1
   // BLOCK_N = 256 staged exists without residual tiles only, and only on request (DRAM_CONV_EPILOGUE_STAGED): AUTO keeps
   // the N = 128 tiling that the bottleneck blocks were tuned with
   const bool staged256 = pl->staged && block_n == 256 && d->res_c == 0 && d->epilogue == DRAM_CONV_EPILOGUE_STAGED;
-  if (pl->staged && block_n > 128 && !staged256) {  // re-tile N: the staged configuration with residual tiles holds BLOCK_N <= 128
-    block_n = 128;
-    pl->block_n = block_n;
-    p.num_n_tiles = d->cout / block_n;
-    const int64_t total2 = (int64_t)p.tiles_per_sample * d->n * p.num_n_tiles;
-    if (total2 > 0x7fffffffLL) {
-      delete pl;
-      set_error("conv3d: too many tiles");
-      return DRAM_E_ARG;
-    }
-    p.total_tiles = (int)total2;
-    pl->n_tiles = p.num_n_tiles;
-    rc = rc == DRAM_OK ? encode_weight_map(&pl->map_w, weight, d->cout, ktot, block_n, epi.is_f16) : rc;
+  if (pl->staged && block_n > 128 && !staged256) block_n = 128;  // the staged configuration with residual tiles holds BLOCK_N <= 128
+  pl->block_n = block_n;
+  const int num_n_tiles = d->cout / block_n;
+
+  // Brick = the tile's work unit.  A brick may fold tn samples: the bricks at the same spatial position of different
+  // samples skip the same padding taps, so with the batch in the brick the spatial extents can be small enough to
+  // line up with a dilated filter's padding.  Auto tiles of filters with more than one tap (1x1x1 ones have no
+  // padding taps; the staged epilogue moves tn = 1 tiles) take the brick with the fewest executed stages.
+  const bool fold = auto_tile && taps > 1 && !pl->staged;
+  const BrickChoice m128 = choose_brick(d, Do, Ho, Wo, BLOCK_M, brick_cost(d, Do, Ho, Wo, tw, th, td, 1), fold);
+  // M256 pair kernel: a brick of 256 voxels, two 128-row boxes.  Unfolded it is two tw x th x td boxes side by side
+  // along the axis that gives the fewest tiles (w first); folded, its halves along the sample axis.
+  BrickChoice pair_base = brick_cost(d, Do, Ho, Wo, 2 * tw, th, td, 1);
+  for (int ax = 1; ax < 3; ++ax) {
+    BrickChoice c = brick_cost(d, Do, Ho, Wo, tw, ax == 1 ? 2 * th : th, ax == 2 ? 2 * td : td, 1);
+    c.split = ax;
+    if (c.tiles < pair_base.tiles) pair_base = c;
   }
+  const BrickChoice m256 = choose_brick(d, Do, Ho, Wo, 2 * BLOCK_M, pair_base, fold);
+  const bool use_pair = !pl->staged && auto_tile &&
+                        pair_plan_wanted(d, block_n, (int64_t)taps * ((d->c1 + d->c2) / BLOCK_K), m256.tiles * num_n_tiles);
+  const BrickChoice &br = use_pair ? m256 : m128;
+
+  pl->kind = 0;
+  ConvKParams &p = pl->p;
+  p.n = d->n; p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.Di = d->di; p.Hi = d->hi; p.Wi = d->wi;
+  p.bw = br.bw; p.bh = br.bh; p.bd = br.bd; p.bn = br.bn;
+  p.tw = br.bw; p.th = br.bh; p.td = br.bd; p.tn = br.bn;
+  if (use_pair) {  // the box is half the brick
+    if (br.split == 3) p.tn = br.bn / 2;
+    else if (br.split == 2) p.td = br.bd / 2;
+    else if (br.split == 1) p.th = br.bh / 2;
+    else p.tw = br.bw / 2;
+  }
+  p.tw_log2 = ilog2(p.tw); p.th_log2 = ilog2(p.th); p.td_log2 = ilog2(p.td);
+  p.tiles_w = ceil_div(Wo, br.bw); p.tiles_h = ceil_div(Ho, br.bh); p.tiles_d = ceil_div(Do, br.bd);
+  p.tiles_per_sample = p.tiles_w * p.tiles_h * p.tiles_d;
+  p.sample_groups = ceil_div(d->n, br.bn);
+  p.num_n_tiles = num_n_tiles;
+  int64_t total = (int64_t)p.tiles_per_sample * p.sample_groups * p.num_n_tiles;
+  if (total > 0x7fffffffLL) {
+    delete pl;
+    set_error("conv3d: too many tiles");
+    return DRAM_E_ARG;
+  }
+  p.total_tiles = (int)total;
+  p.kd = d->kd; p.kh = d->kh; p.kw = d->kw; p.sd = d->sd; p.sh = d->sh; p.sw = d->sw;
+  p.dd = d->dd; p.dh = d->dh; p.dw = d->dw; p.pd = d->pd; p.ph = d->ph; p.pw = d->pw;
+  p.chunks1 = d->c1 / BLOCK_K;
+  p.chunks_total = (d->c1 + d->c2) / BLOCK_K;
+  p.epi = epi;
+  pl->m_tiles = p.tiles_per_sample * p.sample_groups;
+  pl->n_tiles = p.num_n_tiles;
+
+  int rc = encode_act_map(&pl->map_a1, src1, d->n, d->di, d->hi, d->wi, d->c1, BLOCK_K, p.tw, p.th, p.td, d->sw,
+                          d->sh, d->sd, epi.is_f16, p.tn);
+  if (rc == DRAM_OK) {
+    if (d->c2 > 0)
+      rc = encode_act_map(&pl->map_a2, src2, d->n, d->di, d->hi, d->wi, d->c2, BLOCK_K, p.tw, p.th, p.td, d->sw,
+                          d->sh, d->sd, epi.is_f16, p.tn);
+    else
+      pl->map_a2 = pl->map_a1;
+  }
+  if (rc == DRAM_OK) rc = encode_weight_map(&pl->map_w, weight, d->cout, ktot, block_n, epi.is_f16);
   p.staged_res = pl->staged && d->res_c > 0;
   pl->map_out = pl->map_a1;
   pl->map_res = pl->map_a1;
@@ -684,7 +851,7 @@ extern "C" int dram_conv3d_plan_create(const dram_conv_desc *d, const void *src1
         case 256: rc = fill_tile_cfg<256, true>(pl); break;
         default: rc = fill_tile_cfg<128, true>(pl); break;
       }
-    } else if (d->tw == 0 && pair_plan_wanted(d, block_n, (int64_t)taps * p.chunks_total, pl->m_tiles, pl->n_tiles)) {
+    } else if (use_pair) {
       rc = pair_plan_fill(pl);
     } else {
       switch (block_n) {
@@ -695,6 +862,8 @@ extern "C" int dram_conv3d_plan_create(const dram_conv_desc *d, const void *src1
       }
     }
   }
+  p.order = nullptr;
+  pl->order_entries = tile_costs_differ(pl) ? p.total_tiles : 0;
   if (rc != DRAM_OK) {
     delete pl;
     return rc;
@@ -719,19 +888,36 @@ extern "C" int dram_conv3d_plan_info(const dram_conv_plan *plan, int64_t *flops,
   return DRAM_OK;
 }
 
+extern "C" int dram_conv3d_plan_brick(const dram_conv_plan *plan, int32_t *bw, int32_t *bh, int32_t *bd, int32_t *bn,
+                                      int32_t *pair) {
+  DRAM_REQUIRE(plan && bw && bh && bd && bn && pair, "dram_conv3d_plan_brick: null argument");
+  const bool tiles = plan->kind == 0;
+  *bw = tiles ? plan->p.bw : 0;
+  *bh = tiles ? plan->p.bh : 0;
+  *bd = tiles ? plan->p.bd : 0;
+  *bn = tiles ? plan->p.bn : 0;
+  *pair = tiles ? plan->pair : 0;
+  return DRAM_OK;
+}
+
+extern "C" int dram_conv3d_plan_order_size(const dram_conv_plan *plan, int32_t *entries) {
+  DRAM_REQUIRE(plan && entries, "dram_conv3d_plan_order_size: null argument");
+  *entries = plan->order_entries;
+  return DRAM_OK;
+}
+
+extern "C" int dram_conv3d_plan_set_order(dram_conv_plan *plan, int32_t *order, void *stream) {
+  DRAM_REQUIRE(plan && order, "dram_conv3d_plan_set_order: null argument");
+  DRAM_REQUIRE(plan->order_entries > 0, "dram_conv3d_plan_set_order: this plan's tiles all cost the same; it takes no order");
+  conv_tile_order_kernel<<<1, ORDER_THREADS, 0, reinterpret_cast<cudaStream_t>(stream)>>>(plan->p, plan->m_tiles, order);
+  DRAM_CHECK_LAUNCH("conv_tile_order_kernel launch");
+  plan->p.order = order;
+  return DRAM_OK;
+}
+
 // What the kernels actually issue to the tensor pipe: full 128-voxel tiles (border tiles are padded), every
 // non-skipped (tap, chunk) stage at the plan's BLOCK_N — i.e. the algorithmic 2*M*N*K minus the taps skipped in the
 // zero padding plus the tile-quantisation padding.
-static bool host_tap_is_padding(int i0, int extent, int stride, int in_size) {
-  return (i0 + (extent - 1) * stride < 0) || (i0 >= in_size);
-}
-static bool host_brick_tap_skipped(const ConvKParams &p, int m_tile, int zd, int zh, int zw) {
-  const int r = m_tile % p.tiles_per_sample;
-  const int iw = r % p.tiles_w, r2 = r / p.tiles_w, ih = r2 % p.tiles_h, id = r2 / p.tiles_h;
-  return host_tap_is_padding(id * p.td * p.sd + zd * p.dd - p.pd, p.td, p.sd, p.Di) ||
-         host_tap_is_padding(ih * p.th * p.sh + zh * p.dh - p.ph, p.th, p.sh, p.Hi) ||
-         host_tap_is_padding(iw * p.tw * p.sw + zw * p.dw - p.pw, p.tw, p.sw, p.Wi);
-}
 
 extern "C" int dram_conv3d_plan_executed_flops(const dram_conv_plan *plan, int64_t *flops) {
   DRAM_REQUIRE(plan && flops, "dram_conv3d_plan_executed_flops: null argument");
@@ -748,23 +934,9 @@ extern "C" int dram_conv3d_plan_executed_flops(const dram_conv_plan *plan, int64
   }
   const ConvKParams &p = plan->p;
   const int m_tiles = plan->m_tiles;
-  int64_t stages = 0;  // (brick, tap) pairs issued, per n-tile
-  if (plan->pair) {
-    for (int pr = 0; 2 * pr < m_tiles; ++pr)
-      for (int zd = 0; zd < p.kd; ++zd)
-        for (int zh = 0; zh < p.kh; ++zh)
-          for (int zw = 0; zw < p.kw; ++zw) {
-            const bool s0 = host_brick_tap_skipped(p, 2 * pr, zd, zh, zw);
-            const bool s1 = 2 * pr + 1 < m_tiles ? host_brick_tap_skipped(p, 2 * pr + 1, zd, zh, zw) : true;
-            if (!(s0 && s1)) stages += 2;  // both bricks run the MMA when either needs the tap
-          }
-  } else {
-    for (int m = 0; m < m_tiles; ++m)
-      for (int zd = 0; zd < p.kd; ++zd)
-        for (int zh = 0; zh < p.kh; ++zh)
-          for (int zw = 0; zw < p.kw; ++zw)
-            if (!host_brick_tap_skipped(p, m, zd, zh, zw)) ++stages;
-  }
+  int64_t stages = 0;  // (128-row box, tap) pairs issued, per n-tile
+  for (int m = 0; m < m_tiles; ++m) stages += brick_taps(p, m);
+  if (plan->pair) stages *= 2;  // both boxes of a pair brick run the MMA of every tap the brick does not skip
   *flops = 2LL * stages * p.num_n_tiles * 128 * (int64_t)plan->block_n * p.chunks_total * 64;
   return DRAM_OK;
 }

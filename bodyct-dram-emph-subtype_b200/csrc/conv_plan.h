@@ -7,13 +7,14 @@ namespace dram {
 // Per-tap TMA tile kernel (conv3d_umma.cu)
 struct ConvKParams {
   int n, Do, Ho, Wo, Di, Hi, Wi;
-  int tw, th, td;              // tile extents (powers of two, product 128)
-  int tw_log2, th_log2;        // row -> (w,h,d) decode
-  int tiles_w, tiles_h, tiles_d, tiles_per_sample, num_n_tiles, total_tiles;
+  int tw, th, td, tn;          // A box = one 128-row MMA operand: tw x th x td voxels of tn samples (powers of two)
+  int tw_log2, th_log2, td_log2;  // row -> (w,h,d,sample) decode: row = ((s*td + d)*th + h)*tw + w
+  int bw, bh, bd, bn;          // brick = work unit of one tile: the box (M128 kernel) or two boxes (pair kernel)
+  int tiles_w, tiles_h, tiles_d, tiles_per_sample, sample_groups, num_n_tiles, total_tiles;  // bricks along each axis
   int kd, kh, kw, sd, sh, sw, dd, dh, dw, pd, ph, pw;
   int chunks1, chunks_total;   // 64-channel chunks of source 1 / of both sources
   int staged_res;              // staged epilogue: 1 = the residual tile comes through TMA as well
-  int m_tiles_total;           // pair kernel: number of 128-voxel bricks (tiles_per_sample * n)
+  const int *order;            // tile walk order (descending executed stages), or null = tiles in index order
   EpiParams epi;
 };
 
@@ -22,25 +23,36 @@ struct ConvKParams {
 struct TileCoord {
   int n0, sample, d0, h0, w0;
 };
+// Origin of the brick of tile index `tile` (n-tile fastest, then w, h, d, sample group); sample = its first sample.
 __device__ __forceinline__ TileCoord decode_tile(const ConvKParams &p, int tile, int block_n) {
   TileCoord t;
   int n_tile = tile % p.num_n_tiles;
   int m_tile = tile / p.num_n_tiles;
   t.n0 = n_tile * block_n;
-  t.sample = m_tile / p.tiles_per_sample;
-  int r = m_tile - t.sample * p.tiles_per_sample;
+  const int group = m_tile / p.tiles_per_sample;
+  int r = m_tile - group * p.tiles_per_sample;
   int iw = r % p.tiles_w;
   int r2 = r / p.tiles_w;
   int ih = r2 % p.tiles_h;
   int id = r2 / p.tiles_h;
-  t.w0 = iw * p.tw;
-  t.h0 = ih * p.th;
-  t.d0 = id * p.td;
+  t.sample = group * p.bn;
+  t.w0 = iw * p.bw;
+  t.h0 = ih * p.bh;
+  t.d0 = id * p.bd;
   return t;
 }
+// The i-th tile a persistent CTA works on: the plan's cost-sorted permutation when it has one.
+__device__ __forceinline__ int tile_at(const ConvKParams &p, int i) { return p.order ? __ldg(p.order + i) : i; }
+
 // True when every input coordinate the tile reads along one axis for this tap is padding.
 __device__ __forceinline__ bool tap_is_padding(int i0, int extent, int stride, int in_size) {
   return (i0 + (extent - 1) * stride < 0) || (i0 >= in_size);
+}
+// True when the whole brick reads zero padding for this tap; every sample of the brick alike.
+__device__ __forceinline__ bool brick_tap_is_padding(const ConvKParams &p, const TileCoord &t, int zd, int zh, int zw) {
+  return tap_is_padding(t.d0 * p.sd + zd * p.dd - p.pd, p.bd, p.sd, p.Di) ||
+         tap_is_padding(t.h0 * p.sh + zh * p.dh - p.ph, p.bh, p.sh, p.Hi) ||
+         tap_is_padding(t.w0 * p.sw + zw * p.dw - p.pw, p.bw, p.sw, p.Wi);
 }
 #endif
 
@@ -70,7 +82,8 @@ struct dram_conv_plan {
   CUtensorMap map_a1, map_a2, map_w;
   CUtensorMap map_out, map_res;  // staged (TMA store) epilogue of the tile kernel
   int staged;
-  int pair;                      // 1 = M256 kernel (conv3d_pair.cu): two bricks share every weight tile
+  int pair;                      // 1 = M256 kernel (conv3d_pair.cu): two boxes share every weight tile
+  int order_entries;             // entries of the tile order dram_conv3d_plan_set_order writes (0: no order needed)
   dram::ConvKParams p;
   dram::SlabParams sp;
   int block_n;

@@ -415,7 +415,7 @@ __device__ __forceinline__ void epilogue_group_staged(const EpiParams &e, const 
 
 // Host helpers shared by the plan builders (conv3d_umma.cu).
 int encode_act_map(CUtensorMap *map, const void *base, int n, int d, int h, int w, int c, int box_c, int bw,
-                   int bh, int bd, int sw, int sh, int sd, int is_f16);
+                   int bh, int bd, int sw, int sh, int sd, int is_f16, int bn = 1);
 int encode_weight_map(CUtensorMap *map, const void *base, int cout, int64_t ktot, int block_n, int is_f16);
 
 }  // namespace dram

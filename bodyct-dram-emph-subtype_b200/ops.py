@@ -204,6 +204,19 @@ class Conv3dPlan:
         ex = C.c_int64()
         check(lib.dram_conv3d_plan_executed_flops(handle, C.byref(ex)), "dram_conv3d_plan_executed_flops")
         self.executed_flops = ex.value   # tap skipping and tile padding included (what the tensor pipe really does)
+        bw, bh, bd, bn, pair = (C.c_int32() for _ in range(5))
+        check(lib.dram_conv3d_plan_brick(handle, C.byref(bw), C.byref(bh), C.byref(bd), C.byref(bn), C.byref(pair)),
+              "dram_conv3d_plan_brick")
+        self.brick = (bw.value, bh.value, bd.value, bn.value)   # (w, h, d, samples) of a tile; zeros for plane ring
+        self.pair = pair.value != 0                              # M256 kernel: the brick is two 128-row boxes
+        # bricks of different cost (padding skipped at the borders): the kernels walk them by descending cost; the
+        # permutation lives in a caching-allocator buffer and is built on the current stream (capturable, no sync)
+        entries = C.c_int32()
+        check(lib.dram_conv3d_plan_order_size(handle, C.byref(entries)), "dram_conv3d_plan_order_size")
+        self.tile_order = None
+        if entries.value > 0:
+            self.tile_order = torch.empty(entries.value, dtype=torch.int32, device=x1.device)
+            check(lib.dram_conv3d_plan_set_order(handle, _p(self.tile_order), _stream()), "dram_conv3d_plan_set_order")
         self.desc = d
 
     def run(self, max_ctas=0):

@@ -155,6 +155,19 @@ int dram_conv3d_plan_info(const dram_conv_plan *plan, int64_t *flops, int32_t *m
  * 64-channel chunk) stage it executes.  Differs from the algorithmic 2*M*N*K of dram_conv3d_plan_info by the taps
  * skipped inside the zero padding (dilated layers: fewer) and by the padding of border tiles (more). */
 int dram_conv3d_plan_executed_flops(const dram_conv_plan *plan, int64_t *flops);
+/* Work unit of the tile kernels: a brick of bw x bh x bd output voxels of bn samples (bn > 1: the batch is folded
+ * into the brick), run as one 128-row MMA operand or, pair != 0, as two (the M256 kernel).  m_tiles of
+ * dram_conv3d_plan_info counts these bricks.  Plane-ring plans report zeros. */
+int dram_conv3d_plan_brick(const dram_conv_plan *plan, int32_t *bw, int32_t *bh, int32_t *bd, int32_t *bn,
+                           int32_t *pair);
+/* Tile order.  When a plan's bricks execute different numbers of taps (padding skipped at the borders of a dilated
+ * filter), its persistent kernels balance better walking the tiles by descending cost.  order_size gives the int32
+ * entries of that permutation (0: the tiles all cost the same, no order).  set_order builds it on `stream` into the
+ * caller's device buffer `order` (one small kernel; no allocation, no synchronisation, graph-capturable) and makes the
+ * plan's runs walk it; the buffer must stay alive and unchanged until plan_destroy.  Without it the tiles run in index
+ * order, with the same results. */
+int dram_conv3d_plan_order_size(const dram_conv_plan *plan, int32_t *entries);
+int dram_conv3d_plan_set_order(dram_conv_plan *plan, int32_t *order, void *stream);
 /*
  * Work lists (decoder_mask.cu): a run restricted to the work items whose output box, grown by `radius` voxels, meets
  * the support bit mask of dram_decoder_support, whose grid must be the plan's output grid.  Only the 64-channel
